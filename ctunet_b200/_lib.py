@@ -73,6 +73,11 @@ SIGNATURES = {
     "ctu_bn_relu_fwd_train": (I, [I, P, P, D, P, P, P, P, P, F, F, I, P, P, P, I, I, I, I, I, I, P]),
     "ctu_bn_relu_bwd_reduce": (I, [I, P, P, P, P, P, I, I, I, I, I, I, P]),
     "ctu_bn_relu_bwd_apply": (I, [I, P, P, P, P, P, P, D, P, P, P, I, I, I, I, I, I, P]),
+    "ctu_bn_relu_fwd_drop": (I, [I, P, P, P, P, I, I, I, I, I, I, P, P]),
+    "ctu_bn_relu_fwd_train_drop": (I, [I, P, P, D, P, P, P, P, P, F, F, I, P, P, P, I, I, I, I, I, I, P, P]),
+    "ctu_bn_relu_bwd_reduce_drop": (I, [I, P, P, P, P, P, I, I, I, I, I, I, P, P]),
+    "ctu_bn_relu_bwd_apply_drop": (I, [I, P, P, P, P, P, P, D, P, P, P, I, I, I, I, I, I, P, P]),
+    "ctu_dropout3d_keep": (I, [I, P, P, P, I, ULL, P, P, P]),
     "ctu_head_fwd": (I, [I, P, P, I, P, P, I, I, P, P, I, LL, P]),
     "ctu_head_bwd": (I, [I, P, P, I, P, P, I, I, P, P, P, P, P, P, P, I, LL, P]),
     "ctu_head_loss_fwd": (I, [I, P, P, I, P, P, I, I, P, P, I, I, F, F, P, P, P, I, LL, P]),

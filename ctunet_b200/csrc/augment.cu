@@ -11,18 +11,7 @@
 
 namespace ctu {
 
-__device__ __forceinline__ void philox4x32_10(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
-        const uint32_t n0 = hi1 ^ c[1] ^ k0, n2 = hi0 ^ c[3] ^ k1;
-        c[0] = n0, c[1] = lo1, c[2] = n2, c[3] = lo0;
-        k0 += 0x9E3779B9u;
-        k1 += 0xBB67AE85u;
-    }
-}
-
+// (philox4x32_10: common.cuh)
 __device__ __forceinline__ double u53(uint32_t a, uint32_t b) {
     return ((double)(a >> 5) * 67108864.0 + (double)(b >> 6)) / 9007199254740992.0;
 }

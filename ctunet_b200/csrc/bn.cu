@@ -131,6 +131,24 @@ __device__ __forceinline__ V8 bn_relu_apply(const V8& y, const float (&sc)[8], c
     return a;
 }
 
+// Dropout3d after the ReLU (models.py:34,46): a = k * relu(scale*y + shift), k = the keep factor of the (sample, channel),
+// rounded ONCE to the storage type.  The factor multiplies the ReLU output rather than being folded into scale / shift: the
+// backward pass re-elects the pooling arg-max from the unscaled value, and k >= 0 commutes with the max, so the pooled
+// output is MaxPool3d(Dropout3d(a)) as models.py:233 orders them.
+template <typename T>
+__device__ __forceinline__ V8 bn_relu_drop_apply(const V8& y, const float (&sc)[8], const float (&sh)[8], const float (&k)[8]) {
+    V8 a;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) a.v[j] = round_to<T>(k[j] * fmaxf(fmaf(y.v[j], sc[j], sh[j]), 0.f));
+    return a;
+}
+
+// keep factors [n][cpad] of channel block b of sample n (DROP kernels only)
+__device__ __forceinline__ void load_keep(const float* __restrict__ keep, int n, int b, int cpad, float (&k)[8]) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) k[j] = __ldg(keep + (long long)n * cpad + b * 8 + j);
+}
+
 constexpr int kVoxPerThread = 4;   // plain (unpooled) kernels: voxels per thread, strided by the block size
 
 // a = relu(scale*y + shift); grid = (chunks, cb, n)
@@ -202,13 +220,15 @@ __device__ __forceinline__ void bn_scale_shift(const BnFin& f, const float* __re
     }
 }
 
-template <typename T, bool FOLD>
+template <typename T, bool FOLD, bool DROP>
 __global__ void __launch_bounds__(kBnThreads) bn_relu_fwd_kernel(const T* __restrict__ y, const float* __restrict__ ss,
-                                                                 T* __restrict__ a, int cb, long long spatial, BnFin fin) {
+                                                                 T* __restrict__ a, int cb, long long spatial, BnFin fin,
+                                                                 const float* __restrict__ keep) {
     const int b = blockIdx.y, n = blockIdx.z;
     const int cpad = cb * 8;
-    float sc[8], sh[8];
+    float sc[8], sh[8], kf[8];
     bn_scale_shift<FOLD>(fin, ss, b, cpad, blockIdx.x == 0 && n == 0, sc, sh);
+    if constexpr (DROP) load_keep(keep, n, b, cpad, kf);
     const long long base = ((long long)n * cb + b) * spatial;
     const long long s0 = (long long)blockIdx.x * kBnThreads * kVoxPerThread + threadIdx.x;
     V8 v[kVoxPerThread];
@@ -220,7 +240,10 @@ __global__ void __launch_bounds__(kBnThreads) bn_relu_fwd_kernel(const T* __rest
 #pragma unroll
     for (int it = 0; it < kVoxPerThread; ++it) {
         const long long s = s0 + (long long)it * kBnThreads;
-        if (s < spatial) Vec8<T>::store(a + (base + s) * 8, bn_relu_apply<T>(v[it], sc, sh));
+        if (s < spatial) {
+            if constexpr (DROP) Vec8<T>::store(a + (base + s) * 8, bn_relu_drop_apply<T>(v[it], sc, sh, kf));
+            else Vec8<T>::store(a + (base + s) * 8, bn_relu_apply<T>(v[it], sc, sh));
+        }
     }
 }
 
@@ -228,15 +251,18 @@ __global__ void __launch_bounds__(kBnThreads) bn_relu_fwd_kernel(const T* __rest
 //   POOL:  y, a natural [n][cb][d][h][w][8]; pooled = maxpool 2x2x2 of a.
 //   S2D:   y phase-major [n][8*cb][d/2][h/2][w/2][8] (output of the fused up-sampling stage, block = q*cb + b,
 //          q = qd*4 + qh*2 + qw), a natural.
-template <typename T, bool S2D, bool FOLD>
+//   DROP:  a (and pooled) carry the Dropout3d keep factors (natural input only).
+template <typename T, bool S2D, bool FOLD, bool DROP>
 __global__ void __launch_bounds__(kBnThreads) bn_relu_child_fwd_kernel(const T* __restrict__ y,
                                                                        const float* __restrict__ ss, T* __restrict__ a,
                                                                        T* __restrict__ pooled, int cb, int d, int h,
-                                                                       int w, BnFin fin) {
+                                                                       int w, BnFin fin, const float* __restrict__ keep) {
+    static_assert(!(S2D && DROP), "a phase-major BatchNorm input never precedes a dropout site");
     const int b = blockIdx.y, n = blockIdx.z;
     const int cpad = cb * 8;
-    float sc[8], sh[8];
+    float sc[8], sh[8], kf[8];
     bn_scale_shift<FOLD>(fin, ss, b, cpad, blockIdx.x == 0 && n == 0, sc, sh);
+    if constexpr (DROP) load_keep(keep, n, b, cpad, kf);
     const int pd = d / 2, ph = h / 2, pw = w / 2;
     const long long pspatial = (long long)pd * ph * pw;
     const long long ps = (long long)blockIdx.x * kBnThreads + threadIdx.x;
@@ -260,7 +286,9 @@ __global__ void __launch_bounds__(kBnThreads) bn_relu_child_fwd_kernel(const T* 
 #pragma unroll
     for (int q = 0; q < 8; ++q) {
         const int z = 2 * pz + (q >> 2), yy = 2 * py + ((q >> 1) & 1), x = 2 * px + (q & 1);
-        V8 r = bn_relu_apply<T>(in[q], sc, sh);
+        V8 r;
+        if constexpr (DROP) r = bn_relu_drop_apply<T>(in[q], sc, sh, kf);
+        else r = bn_relu_apply<T>(in[q], sc, sh);
         Vec8<T>::store(a + (base + ((long long)z * h + yy) * w + x) * 8, r);
         if (!S2D) {
 #pragma unroll
@@ -272,6 +300,8 @@ __global__ void __launch_bounds__(kBnThreads) bn_relu_child_fwd_kernel(const T* 
 
 // ---------------------------------------------------------------------------- backward
 // Gradient entering the BatchNorm output: dz = (dA + [child is the first max of its window] * dP) * [a > 0].
+// DROP: dz = k * (dA + [winner] * dP) * [scale*y + shift > 0] with the keep factors of the forward (the batch statistics
+// stay those of y: BatchNorm comes before the dropout).
 // MODE 0: one voxel at a time (kVoxPerThread per thread); MODE 1 (pool): the 8 children of one pooled voxel;
 // MODE 2 (s2d): the 8 children of one low-res voxel with y / dy phase-major and dA natural.
 struct BwdArgs {
@@ -281,6 +311,7 @@ struct BwdArgs {
     const void* dA;
     const void* dP;
     double* sums2;        // reduce: output; apply: input
+    const float* keep;    // Dropout3d keep factors [n][cpad] (DROP kernels)
     double count;
     void* dy;
     float* dgamma;
@@ -289,9 +320,10 @@ struct BwdArgs {
     long long nblk;       // chunks of kBnThreads (x kVoxPerThread in mode 0) voxels per (n, block) plane
 };
 
-template <typename T, int MODE, bool APPLY>
+template <typename T, int MODE, bool APPLY, bool DROP>
 __global__ void __launch_bounds__(kBnThreads, 2) bn_relu_bwd_kernel(BwdArgs p) {
     constexpr bool POOL = MODE == 1, S2D = MODE == 2;     // MODE 3: the child structure on a natural, unpooled tensor
+    static_assert(!(S2D && DROP), "a phase-major BatchNorm input never precedes a dropout site");
     const int b = blockIdx.y, n = blockIdx.z;
     const int cpad = p.cb * 8;
     __shared__ float kk[16];
@@ -306,7 +338,8 @@ __global__ void __launch_bounds__(kBnThreads, 2) bn_relu_bwd_kernel(BwdArgs p) {
         }
         __syncthreads();
     }
-    float sc[8], sh[8], mean[8], invstd[8], k1[8], k2[8];
+    float sc[8], sh[8], mean[8], invstd[8], k1[8], k2[8], kf[8];
+    if constexpr (DROP) load_keep(p.keep, n, b, cpad, kf);
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
         sc[j] = __ldg(p.ss + b * 8 + j);
@@ -350,7 +383,7 @@ __global__ void __launch_bounds__(kBnThreads, 2) bn_relu_bwd_kernel(BwdArgs p) {
 #pragma unroll
                 for (int j = 0; j < 8; ++j) {
                     const float av = fmaf(yv[it].v[j], sc[j], sh[j]);
-                    const float dz = av > 0.f ? g[it].v[j] : 0.f;
+                    const float dz = av > 0.f ? (DROP ? kf[j] * g[it].v[j] : g[it].v[j]) : 0.f;
                     const float xhat = (yv[it].v[j] - mean[j]) * invstd[j];
                     if (APPLY) {
                         o.v[j] = sc[j] * (dz - k1[j] - xhat * k2[j]);
@@ -438,6 +471,7 @@ __global__ void __launch_bounds__(kBnThreads, 2) bn_relu_bwd_kernel(BwdArgs p) {
                 for (int j = 0; j < 8; ++j) {
                     float dz = g.v[j];
                     if (POOL) dz += (win[j] == q) ? gp.v[j] : 0.f;
+                    if constexpr (DROP) dz *= kf[j];
                     dz = fmaf(yq.v[j], sc[j], sh[j]) > 0.f ? dz : 0.f;
                     const float xhat = (yq.v[j] - mean[j]) * invstd[j];
                     if (APPLY) {
@@ -507,9 +541,12 @@ int ctu_bn_running_update(const double* sums, double count, float* running_mean,
 }
 
 static int bn_relu_fwd_launch(int dtype, const void* y, const float* ss, void* a, void* pooled, int c, int n, int d, int h,
-                              int w, int y_phase_major, const BnFin& fin, ctu_stream stream, const char* what) {
+                              int w, int y_phase_major, const BnFin& fin, const float* keep, ctu_stream stream,
+                              const char* what) {
     CTU_REQUIRE(y && (ss || fin.sums) && a && c > 0 && n > 0 && d > 0 && h > 0 && w > 0, "%s: bad arguments", what);
     CTU_REQUIRE(!(y_phase_major && pooled), "%s: a phase-major input is never pooled", what);
+    CTU_REQUIRE(!(y_phase_major && keep), "%s: a phase-major input never carries dropout keep factors", what);
+    const bool drop = keep != nullptr;
     const int cb = (c + 7) / 8;
     const long long spatial = (long long)d * h * w;
     const bool fold = fin.sums != nullptr;
@@ -518,34 +555,53 @@ static int bn_relu_fwd_launch(int dtype, const void* y, const float* ss, void* a
         CTU_REQUIRE(d % 2 == 0 && h % 2 == 0 && w % 2 == 0, "%s: needs even dims (%d,%d,%d)", what, d, h, w);
         dim3 grid(cdiv(spatial / 8, kBnThreads), cb, n);
         CTU_DISPATCH_DTYPE(dtype, {
-            if (y_phase_major && fold) bn_relu_child_fwd_kernel<T, true, true><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, nullptr, cb, d, h, w, fin);
-            else if (y_phase_major) bn_relu_child_fwd_kernel<T, true, false><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, nullptr, cb, d, h, w, fin);
-            else if (fold) bn_relu_child_fwd_kernel<T, false, true><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, (T*)pooled, cb, d, h, w, fin);
-            else bn_relu_child_fwd_kernel<T, false, false><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, (T*)pooled, cb, d, h, w, fin);
+            if (y_phase_major && fold) bn_relu_child_fwd_kernel<T, true, true, false><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, nullptr, cb, d, h, w, fin, nullptr);
+            else if (y_phase_major) bn_relu_child_fwd_kernel<T, true, false, false><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, nullptr, cb, d, h, w, fin, nullptr);
+            else if (fold && drop) bn_relu_child_fwd_kernel<T, false, true, true><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, (T*)pooled, cb, d, h, w, fin, keep);
+            else if (drop) bn_relu_child_fwd_kernel<T, false, false, true><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, (T*)pooled, cb, d, h, w, fin, keep);
+            else if (fold) bn_relu_child_fwd_kernel<T, false, true, false><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, (T*)pooled, cb, d, h, w, fin, nullptr);
+            else bn_relu_child_fwd_kernel<T, false, false, false><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, (T*)pooled, cb, d, h, w, fin, nullptr);
         });
     } else {
         dim3 grid(cdiv(spatial, kBnThreads * kVoxPerThread), cb, n);
         CTU_DISPATCH_DTYPE(dtype, {
-            if (fold) bn_relu_fwd_kernel<T, true><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, cb, spatial, fin);
-            else bn_relu_fwd_kernel<T, false><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, cb, spatial, fin);
+            if (fold && drop) bn_relu_fwd_kernel<T, true, true><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, cb, spatial, fin, keep);
+            else if (drop) bn_relu_fwd_kernel<T, false, true><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, cb, spatial, fin, keep);
+            else if (fold) bn_relu_fwd_kernel<T, true, false><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, cb, spatial, fin, nullptr);
+            else bn_relu_fwd_kernel<T, false, false><<<grid, kBnThreads, 0, st>>>((const T*)y, ss, (T*)a, cb, spatial, fin, nullptr);
         });
     }
     return check_launch(what);
 }
 
+int ctu_bn_relu_fwd_drop(int dtype, const void* y, const float* ss, void* a, void* pooled, int c, int n, int d, int h,
+                         int w, int y_phase_major, const float* keep, ctu_stream stream) {
+    BnFin fin = {};
+    return bn_relu_fwd_launch(dtype, y, ss, a, pooled, c, n, d, h, w, y_phase_major, fin, keep, stream,
+                              keep ? "ctu_bn_relu_fwd_drop" : "ctu_bn_relu_fwd");
+}
+
 int ctu_bn_relu_fwd(int dtype, const void* y, const float* ss, void* a, void* pooled, int c, int n, int d, int h, int w,
                     int y_phase_major, ctu_stream stream) {
-    BnFin fin = {};
-    return bn_relu_fwd_launch(dtype, y, ss, a, pooled, c, n, d, h, w, y_phase_major, fin, stream, "ctu_bn_relu_fwd");
+    return ctu_bn_relu_fwd_drop(dtype, y, ss, a, pooled, c, n, d, h, w, y_phase_major, nullptr, stream);
+}
+
+int ctu_bn_relu_fwd_train_drop(int dtype, const void* y, const double* sums, double count, const float* gamma,
+                               const float* beta, float* running_mean, float* running_var, long long* num_batches_tracked,
+                               float momentum, float eps, int n_updates, float* ss, void* a, void* pooled, int c, int n,
+                               int d, int h, int w, int y_phase_major, const float* keep, ctu_stream stream) {
+    const char* what = keep ? "ctu_bn_relu_fwd_train_drop" : "ctu_bn_relu_fwd_train";
+    CTU_REQUIRE(sums && gamma && beta && ss && count > 0, "%s: bad arguments", what);
+    BnFin fin = {sums, count, gamma, beta, running_mean, running_var, num_batches_tracked, momentum, eps, c, n_updates, ss};
+    return bn_relu_fwd_launch(dtype, y, ss, a, pooled, c, n, d, h, w, y_phase_major, fin, keep, stream, what);
 }
 
 int ctu_bn_relu_fwd_train(int dtype, const void* y, const double* sums, double count, const float* gamma, const float* beta,
                           float* running_mean, float* running_var, long long* num_batches_tracked, float momentum, float eps,
                           int n_updates, float* ss, void* a, void* pooled, int c, int n, int d, int h, int w,
                           int y_phase_major, ctu_stream stream) {
-    CTU_REQUIRE(sums && gamma && beta && ss && count > 0, "ctu_bn_relu_fwd_train: bad arguments");
-    BnFin fin = {sums, count, gamma, beta, running_mean, running_var, num_batches_tracked, momentum, eps, c, n_updates, ss};
-    return bn_relu_fwd_launch(dtype, y, ss, a, pooled, c, n, d, h, w, y_phase_major, fin, stream, "ctu_bn_relu_fwd_train");
+    return ctu_bn_relu_fwd_train_drop(dtype, y, sums, count, gamma, beta, running_mean, running_var, num_batches_tracked,
+                                      momentum, eps, n_updates, ss, a, pooled, c, n, d, h, w, y_phase_major, nullptr, stream);
 }
 
 static int bn_bwd(int dtype, BwdArgs& p, int n, bool apply, int y_phase_major, cudaStream_t stream, const char* what) {
@@ -563,6 +619,11 @@ static int bn_bwd(int dtype, BwdArgs& p, int n, bool apply, int y_phase_major, c
         set_error("%s: missing gradient", what);
         return CTU_ERR_INVALID;
     }
+    if (y_phase_major && p.keep) {
+        set_error("%s: a phase-major BatchNorm input never carries dropout keep factors", what);
+        return CTU_ERR_INVALID;
+    }
+    const bool drop = p.keep != nullptr;
     // unpooled natural tensors with even dims also take the 8-children-per-thread structure (mode 3): measured 2x
     // faster than the strided one-voxel-at-a-time loop of mode 0
     const bool even = !(p.d % 2 || p.h % 2 || p.w % 2);
@@ -576,42 +637,66 @@ static int bn_bwd(int dtype, BwdArgs& p, int n, bool apply, int y_phase_major, c
     }
     dim3 grid((unsigned)gx, p.cb, n);
     CTU_DISPATCH_DTYPE(dtype, {
-        if (mode == 1 && apply) bn_relu_bwd_kernel<T, 1, true><<<grid, kBnThreads, 0, stream>>>(p);
-        else if (mode == 1) bn_relu_bwd_kernel<T, 1, false><<<grid, kBnThreads, 0, stream>>>(p);
-        else if (mode == 2 && apply) bn_relu_bwd_kernel<T, 2, true><<<grid, kBnThreads, 0, stream>>>(p);
-        else if (mode == 2) bn_relu_bwd_kernel<T, 2, false><<<grid, kBnThreads, 0, stream>>>(p);
-        else if (mode == 3 && apply) bn_relu_bwd_kernel<T, 3, true><<<grid, kBnThreads, 0, stream>>>(p);
-        else if (mode == 3) bn_relu_bwd_kernel<T, 3, false><<<grid, kBnThreads, 0, stream>>>(p);
-        else if (apply) bn_relu_bwd_kernel<T, 0, true><<<grid, kBnThreads, 0, stream>>>(p);
-        else bn_relu_bwd_kernel<T, 0, false><<<grid, kBnThreads, 0, stream>>>(p);
+        if (drop) {
+            if (mode == 1 && apply) bn_relu_bwd_kernel<T, 1, true, true><<<grid, kBnThreads, 0, stream>>>(p);
+            else if (mode == 1) bn_relu_bwd_kernel<T, 1, false, true><<<grid, kBnThreads, 0, stream>>>(p);
+            else if (mode == 3 && apply) bn_relu_bwd_kernel<T, 3, true, true><<<grid, kBnThreads, 0, stream>>>(p);
+            else if (mode == 3) bn_relu_bwd_kernel<T, 3, false, true><<<grid, kBnThreads, 0, stream>>>(p);
+            else if (apply) bn_relu_bwd_kernel<T, 0, true, true><<<grid, kBnThreads, 0, stream>>>(p);
+            else bn_relu_bwd_kernel<T, 0, false, true><<<grid, kBnThreads, 0, stream>>>(p);
+        }
+        else if (mode == 1 && apply) bn_relu_bwd_kernel<T, 1, true, false><<<grid, kBnThreads, 0, stream>>>(p);
+        else if (mode == 1) bn_relu_bwd_kernel<T, 1, false, false><<<grid, kBnThreads, 0, stream>>>(p);
+        else if (mode == 2 && apply) bn_relu_bwd_kernel<T, 2, true, false><<<grid, kBnThreads, 0, stream>>>(p);
+        else if (mode == 2) bn_relu_bwd_kernel<T, 2, false, false><<<grid, kBnThreads, 0, stream>>>(p);
+        else if (mode == 3 && apply) bn_relu_bwd_kernel<T, 3, true, false><<<grid, kBnThreads, 0, stream>>>(p);
+        else if (mode == 3) bn_relu_bwd_kernel<T, 3, false, false><<<grid, kBnThreads, 0, stream>>>(p);
+        else if (apply) bn_relu_bwd_kernel<T, 0, true, false><<<grid, kBnThreads, 0, stream>>>(p);
+        else bn_relu_bwd_kernel<T, 0, false, false><<<grid, kBnThreads, 0, stream>>>(p);
     });
     return check_launch(what);
 }
 
-int ctu_bn_relu_bwd_reduce(int dtype, const void* y, const float* ss, const void* dA, const void* dP, double* sums2,
-                           int c, int n, int d, int h, int w, int y_phase_major, ctu_stream stream) {
+int ctu_bn_relu_bwd_reduce_drop(int dtype, const void* y, const float* ss, const void* dA, const void* dP, double* sums2,
+                                int c, int n, int d, int h, int w, int y_phase_major, const float* keep, ctu_stream stream) {
+    const char* what = keep ? "ctu_bn_relu_bwd_reduce_drop" : "ctu_bn_relu_bwd_reduce";
     const bool prezeroed = (y_phase_major & CTU_ACCUM_PREZEROED) != 0;
     y_phase_major &= ~CTU_ACCUM_PREZEROED;
-    CTU_REQUIRE(y && ss && sums2 && (dA || dP) && c > 0 && n > 0 && d > 0 && h > 0 && w > 0, "ctu_bn_relu_bwd_reduce: bad arguments");
+    CTU_REQUIRE(y && ss && sums2 && (dA || dP) && c > 0 && n > 0 && d > 0 && h > 0 && w > 0, "%s: bad arguments", what);
     BwdArgs p = {};
     p.y = y; p.ss = ss; p.dA = dA; p.dP = dP; p.sums2 = sums2; p.c = c; p.cb = (c + 7) / 8; p.d = d; p.h = h; p.w = w;
+    p.keep = keep;
     cudaError_t e = prezeroed ? cudaSuccess : cudaMemsetAsync(sums2, 0, sizeof(double) * 2 * p.cb * 8, (cudaStream_t)stream);
     if (e != cudaSuccess) {
-        set_error("ctu_bn_relu_bwd_reduce: memset: %s", cudaGetErrorString(e));
+        set_error("%s: memset: %s", what, cudaGetErrorString(e));
         return (int)e;
     }
-    return bn_bwd(dtype, p, n, false, y_phase_major, (cudaStream_t)stream, "ctu_bn_relu_bwd_reduce");
+    return bn_bwd(dtype, p, n, false, y_phase_major, (cudaStream_t)stream, what);
+}
+
+int ctu_bn_relu_bwd_reduce(int dtype, const void* y, const float* ss, const void* dA, const void* dP, double* sums2,
+                           int c, int n, int d, int h, int w, int y_phase_major, ctu_stream stream) {
+    return ctu_bn_relu_bwd_reduce_drop(dtype, y, ss, dA, dP, sums2, c, n, d, h, w, y_phase_major, nullptr, stream);
+}
+
+int ctu_bn_relu_bwd_apply_drop(int dtype, const void* y, const float* ss, const float* gamma, const void* dA, const void* dP,
+                               const double* sums2, double count, void* dy, float* dgamma, float* dbeta, int c, int n, int d,
+                               int h, int w, int y_phase_major, const float* keep, ctu_stream stream) {
+    const char* what = keep ? "ctu_bn_relu_bwd_apply_drop" : "ctu_bn_relu_bwd_apply";
+    CTU_REQUIRE(y && ss && sums2 && dy && dgamma && dbeta && (dA || dP) && count > 0 && c > 0 && n > 0 && d > 0 && h > 0 && w > 0,
+                "%s: bad arguments", what);
+    BwdArgs p = {};
+    p.y = y; p.ss = ss; p.gamma = gamma; p.dA = dA; p.dP = dP; p.sums2 = const_cast<double*>(sums2); p.count = count;
+    p.dy = dy; p.dgamma = dgamma; p.dbeta = dbeta; p.c = c; p.cb = (c + 7) / 8; p.d = d; p.h = h; p.w = w;
+    p.keep = keep;
+    return bn_bwd(dtype, p, n, true, y_phase_major, (cudaStream_t)stream, what);
 }
 
 int ctu_bn_relu_bwd_apply(int dtype, const void* y, const float* ss, const float* gamma, const void* dA, const void* dP,
                           const double* sums2, double count, void* dy, float* dgamma, float* dbeta, int c, int n, int d,
                           int h, int w, int y_phase_major, ctu_stream stream) {
-    CTU_REQUIRE(y && ss && sums2 && dy && dgamma && dbeta && (dA || dP) && count > 0 && c > 0 && n > 0 && d > 0 && h > 0 && w > 0,
-                "ctu_bn_relu_bwd_apply: bad arguments");
-    BwdArgs p = {};
-    p.y = y; p.ss = ss; p.gamma = gamma; p.dA = dA; p.dP = dP; p.sums2 = const_cast<double*>(sums2); p.count = count;
-    p.dy = dy; p.dgamma = dgamma; p.dbeta = dbeta; p.c = c; p.cb = (c + 7) / 8; p.d = d; p.h = h; p.w = w;
-    return bn_bwd(dtype, p, n, true, y_phase_major, (cudaStream_t)stream, "ctu_bn_relu_bwd_apply");
+    return ctu_bn_relu_bwd_apply_drop(dtype, y, ss, gamma, dA, dP, sums2, count, dy, dgamma, dbeta, c, n, d, h, w,
+                                      y_phase_major, nullptr, stream);
 }
 
 }  // extern "C"

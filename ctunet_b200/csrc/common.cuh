@@ -133,6 +133,20 @@ template <> __device__ __forceinline__ float round_to<__nv_bfloat16>(float x) {
     return __bfloat162float(__float2bfloat16_rn(x));
 }
 
+// Counter-based Philox4x32-10 (Salmon et al., SC'11): 128 random bits per (counter c, key k0:k1), no state to carry
+// between launches.  Used by the salt-and-pepper noise (augment.cu) and the Dropout3d keep factors (dropout.cu).
+__device__ __forceinline__ void philox4x32_10(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
+        const uint32_t n0 = hi1 ^ c[1] ^ k0, n2 = hi0 ^ c[3] ^ k1;
+        c[0] = n0, c[1] = lo1, c[2] = n2, c[3] = lo0;
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -83,7 +83,8 @@ WGRAD_ARENA = os.environ.get("CTU_WGRAD_ARENA", "0") == "1"     # (measured: 4.2
 WACC_CHUNK_FLOATS = 4 * 1024 * 1024
 CONVT_WGRAD_ASYNC = os.environ.get("CTU_CONVT_WGRAD_ASYNC", "0") == "1"
 WGRAD_AFTER_DGRAD = int(os.environ.get("CTU_WGRAD_AFTER", "2"))      # 0 never, 1 always, 2 only for stages with >= 2 data gradients
-_SIDE_HIGH = (0,)          # which: 0 weight preparation, 1 weight gradients, 2 dead branch, 3 network-input gradient
+_SIDE_HIGH = (0, 5)        # which: 0 weight preparation, 1 weight gradients, 2 dead branch, 3 network-input gradient,
+                           # 4 leaf tails, 5 Dropout3d keep factors
 
 
 def _side_stream(device, which=0):
@@ -128,6 +129,35 @@ class Act:
         return self.buf.data_ptr()
 
 
+_U64 = (1 << 64) - 1
+
+
+def _splitmix64(x: int) -> int:
+    x = (x + 0x9E3779B97F4A7C15) & _U64
+    x = ((x ^ (x >> 30)) * 0xBF58476D1CE4E5B9) & _U64
+    x = ((x ^ (x >> 27)) * 0x94D049BB133111EB) & _U64
+    return x ^ (x >> 31)
+
+
+class DropoutRNG:
+    """Random state of the Dropout3d sites of one model on one device: a 64-bit Philox key and the pass counter, which
+    lives in device memory and is advanced by the mask launch itself (ctu_dropout3d_keep), so a captured step draws new
+    masks on every replay.  The key is ``torch.initial_seed()`` at creation (``torch.manual_seed(s)`` reproduces a run),
+    mixed with the device index (``nn.DataParallel`` replicas) and the ``torch.distributed`` rank when one is initialised,
+    so replicas and ranks draw independent masks."""
+    __slots__ = ("key", "counter", "last")
+
+    def __init__(self, device):
+        device = torch.device(device)
+        rank = 0
+        if torch.distributed.is_available() and torch.distributed.is_initialized():
+            rank = torch.distributed.get_rank()
+        idx = device.index if device.index is not None else torch.cuda.current_device()
+        self.key = _splitmix64(torch.initial_seed() ^ _splitmix64((idx << 32) | (rank & 0xFFFFFFFF)))
+        self.counter = torch.zeros(1, dtype=torch.int64, device=device)
+        self.last = {}          # site name -> [N, C] view of the keep factors of the last pass that drew masks
+
+
 class Engine:
     def __init__(self, device, compute_dtype: str, record: bool):
         if compute_dtype not in ("bf16", "fp32"):
@@ -167,6 +197,7 @@ class Engine:
         # gather, (labels, origins, patch, dims) makes the head write hard labels (scattered at the origins when given)
         self.patch_src = None
         self.label_dst = None
+        self._keep_event = None                    # Dropout3d keep factors drawn on their own stream (see dropout_masks)
 
     # ------------------------------------------------------------------ weight preparation on a side stream
     def begin(self, store: dict, key) -> None:
@@ -227,6 +258,36 @@ class Engine:
         if self._dead_stream is not None:
             torch.cuda.current_stream().wait_stream(self._dead_stream)
             self._dead_stream = None
+        self._wait_keep()                            # (masks nobody applied: still joined, e.g. for a graph capture)
+
+    # ------------------------------------------------------------------ Dropout3d keep factors
+    def dropout_masks(self, rng: DropoutRNG, n: int, sites):
+        """Draw the keep factors of every active Dropout3d site of this pass in ONE launch on a side stream (they depend on
+        nothing but the random state, so they are off the layer chain).  ``sites``: [(site id, channels, p)]; returns one
+        float32 [n, cpad] tensor per site.  The first BatchNorm stage that applies them waits for the launch."""
+        cpads = [(c + 7) // 8 * 8 for _, c, _ in sites]
+        main = torch.cuda.current_stream()
+        side = _side_stream(self.device, 5)
+        side.wait_stream(main)
+        with torch.cuda.stream(side):
+            buf = self.f32(n * sum(cpads))
+            call("ctu_dropout3d_keep", len(sites), int_array([s[0] for s in sites]), int_array([s[1] for s in sites]),
+                 (_lib.c_float * len(sites))(*[float(s[2]) for s in sites]), n, rng.key, rng.counter.data_ptr(),
+                 buf.data_ptr(), stream_ptr())
+            ev = torch.cuda.Event()
+            ev.record(side)
+        buf.record_stream(main)
+        self._keep_event = ev
+        out, off = [], 0
+        for cp in cpads:
+            out.append(buf[off:off + n * cp].view(n, cp))
+            off += n * cp
+        return out
+
+    def _wait_keep(self):
+        if self._keep_event is not None:
+            torch.cuda.current_stream().wait_event(self._keep_event)
+            self._keep_event = None
 
     def off_critical_path(self, *inputs: "Act"):
         """Context: run stages whose OUTPUT nobody consumes (the generic UNet's discarded center block,
@@ -579,7 +640,7 @@ class Engine:
                 dx = self.new_act(s.c, s.n, s.d, s.h, s.w)
                 info = s.bn
                 if (BN_BWD_FUSE and info is not None and info["consumers"] == 1 and not info["pool"] and tc_d[i] == 1
-                        and self.dtype == CTU_BF16
+                        and self.dtype == CTU_BF16 and not info["drop"]
                         and lib.ctu_conv_tc_bnred_supported(k, 1, int_array([cout]), s.c, s.d, s.h, s.w)):
                     # dx is dA of a BatchNorm+ReLU stage consumed only here: its backward reductions ride in this epilogue
                     sums2 = self.f64(2 * ((s.c + 7) // 8 * 8))
@@ -797,9 +858,12 @@ class Engine:
         return y
 
     # ------------------------------------------------------------------ BatchNorm3d + ReLU (+ MaxPool)
-    def bn_relu(self, y: Act, bn, training: bool, extra_updates: int = 0, pool: bool = False):
+    def bn_relu(self, y: Act, bn, training: bool, extra_updates: int = 0, pool: bool = False, keep=None):
         """Returns ``a`` or ``(a, pooled)``.  ``extra_updates``: additional running-stat updates applied
-        when the backward pass runs (the reentrant-checkpoint recomputation of the reference)."""
+        when the backward pass runs (the reentrant-checkpoint recomputation of the reference).  ``keep``: the float32
+        [n, cpad] keep factors of the Dropout3d that follows the ReLU (``dropout_masks``), applied inside the kernels and
+        kept for the backward pass: the reference's reentrant checkpoint restores the RNG state, so its recomputation draws
+        the same mask and reusing the forward's factors is exact."""
         # nn.BatchNorm3d configurations no preset of the reference uses (models.py:27,31 build BatchNorm3d(c) with the
         # defaults) are refused rather than silently computed differently from torch:
         if bn.momentum is None:
@@ -836,22 +900,37 @@ class Engine:
         # one launch less on the critical path.  Large ones keep the separate 1-block finalize: the per-block prologue
         # (double-precision divide / sqrt + a barrier) costs the short-lived blocks of a 128^3 launch 17 us (ncu: 38 -> 56 us).
         fold = training and yn * yd * yh * yw <= BN_FOLD_MAX_VOXELS
+        kp = None
+        if keep is not None:
+            if pm:
+                raise RuntimeError("internal: a phase-major BatchNorm input never precedes a dropout site")
+            self._wait_keep()
+            kp = keep.data_ptr()
         if training and not fold:
             call("ctu_bn_finalize", sums.data_ptr(), count, bn.weight.data_ptr(), bn.bias.data_ptr(),
                  bn.running_mean.data_ptr() if track else None, bn.running_var.data_ptr() if track else None,
                  bn.num_batches_tracked.data_ptr() if track else None, mom, float(bn.eps), c, 1, 1, ss.data_ptr(), st)
-        if fold:
+        if fold and kp is not None:
+            call("ctu_bn_relu_fwd_train_drop", self.dtype, y.ptr, sums.data_ptr(), count, bn.weight.data_ptr(),
+                 bn.bias.data_ptr(), bn.running_mean.data_ptr() if track else None,
+                 bn.running_var.data_ptr() if track else None, bn.num_batches_tracked.data_ptr() if track else None, mom,
+                 float(bn.eps), 1, ss.data_ptr(), a.ptr, pooled.ptr if pool else None, c, yn, yd, yh, yw, pm, kp, st)
+        elif fold:
             call("ctu_bn_relu_fwd_train", self.dtype, y.ptr, sums.data_ptr(), count, bn.weight.data_ptr(), bn.bias.data_ptr(),
                  bn.running_mean.data_ptr() if track else None, bn.running_var.data_ptr() if track else None,
                  bn.num_batches_tracked.data_ptr() if track else None, mom, float(bn.eps), 1, ss.data_ptr(), a.ptr,
                  pooled.ptr if pool else None, c, yn, yd, yh, yw, pm, st)
+        elif kp is not None:
+            call("ctu_bn_relu_fwd_drop", self.dtype, y.ptr, ss.data_ptr(), a.ptr, pooled.ptr if pool else None,
+                 c, yn, yd, yh, yw, pm, kp, st)
         else:
             call("ctu_bn_relu_fwd", self.dtype, y.ptr, ss.data_ptr(), a.ptr, pooled.ptr if pool else None,
                  c, yn, yd, yh, yw, pm, st)
         if self.record:
             if not training:
                 raise RuntimeError("backward through eval-mode BatchNorm is not supported by the fused path")
-            a.bn = {"y": y, "ss": ss, "pm": pm, "pool": bool(pool), "consumers": 0, "sums2": None}
+            # (a dropout stage never takes the reduction in the consumer's epilogue: that epilogue knows nothing of keep)
+            a.bn = {"y": y, "ss": ss, "pm": pm, "pool": bool(pool), "drop": kp is not None, "consumers": 0, "sums2": None}
 
             def bwd():
                 dA = self.agrads.pop(id(a), None)
@@ -885,14 +964,23 @@ class Engine:
                 pP = dP.ptr if dP is not None else None
                 sums2 = a.bn["sums2"]
                 a.bn = None                                           # (drop the reference cycle through the closure)
-                if sums2 is None or dP is not None:                  # not produced by the consumer's epilogue: reduce here
+                kq = keep.data_ptr() if keep is not None else None      # (the closure holds the keep factors alive)
+                if kq is not None:
+                    sums2 = self.acc64(2 * cpad)
+                    call("ctu_bn_relu_bwd_reduce_drop", self.dtype, y.ptr, ss.data_ptr(), pA, pP, sums2.data_ptr(),
+                         c, yn, yd, yh, yw, pm | self._pz(sums2), kq, st)
+                elif sums2 is None or dP is not None:                # not produced by the consumer's epilogue: reduce here
                     sums2 = self.acc64(2 * cpad)
                     call("ctu_bn_relu_bwd_reduce", self.dtype, y.ptr, ss.data_ptr(), pA, pP, sums2.data_ptr(),
                          c, yn, yd, yh, yw, pm | self._pz(sums2), st)
                 dy = self.new_act(y.c, y.n, y.d, y.h, y.w)          # same layout as y (phase-major stays phase-major)
                 dg, db = self._grad_buffer(bn.weight), self._grad_buffer(bn.bias)
-                call("ctu_bn_relu_bwd_apply", self.dtype, y.ptr, ss.data_ptr(), bn.weight.data_ptr(), pA, pP,
-                     sums2.data_ptr(), count, dy.ptr, dg.data_ptr(), db.data_ptr(), c, yn, yd, yh, yw, pm, st)
+                if kq is not None:
+                    call("ctu_bn_relu_bwd_apply_drop", self.dtype, y.ptr, ss.data_ptr(), bn.weight.data_ptr(), pA, pP,
+                         sums2.data_ptr(), count, dy.ptr, dg.data_ptr(), db.data_ptr(), c, yn, yd, yh, yw, pm, kq, st)
+                else:
+                    call("ctu_bn_relu_bwd_apply", self.dtype, y.ptr, ss.data_ptr(), bn.weight.data_ptr(), pA, pP,
+                         sums2.data_ptr(), count, dy.ptr, dg.data_ptr(), db.data_ptr(), c, yn, yd, yh, yw, pm, st)
                 self._add_pgrad(bn.weight, dg)
                 self._add_pgrad(bn.bias, db)
                 self._set_agrad(y, dy)

@@ -14,7 +14,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from .engine import Engine
+from .engine import DropoutRNG, Engine
 
 _COMPUTE_DTYPE = "bf16"
 
@@ -122,6 +122,49 @@ class _FusedNet(nn.Module):
     def _run(self, eng: Engine, x: torch.Tensor, training: bool):
         raise NotImplementedError
 
+    # ---- Dropout3d (the last module of every block, models.py:34,46,97,411,438,492)
+    def _dropout_sites(self):
+        """[(name, nn.Dropout3d, channels)] of the dropout sites whose input the network uses, in a fixed order: the index
+        is the site's number in the Philox counter of its keep factors (csrc/dropout.cu)."""
+        raise NotImplementedError
+
+    def _active_dropout(self):
+        """Sites that drop in this pass: read from each site's own module like torch does (``.training`` and ``.p``), so
+        an eval-mode net with its Dropout3d modules switched to train draws masks too (Monte-Carlo dropout inference)."""
+        return [(i, name, m, c) for i, (name, m, c) in enumerate(self._dropout_sites()) if m.training and m.p > 0]
+
+    def _dropout_config(self):
+        """What a captured graph / weight-preparation plan of a pass depends on: (site, p) of every active site."""
+        return tuple((i, float(m.p)) for i, _, m, _ in self._active_dropout())
+
+    def _draw_dropout(self, eng: Engine, n: int):
+        """Keep factors of every active site for this pass (one launch beside the layer chain): {site name: [n, cpad]}."""
+        act = self._active_dropout()
+        if not act:
+            return {}
+        # a plain attribute, not a buffer: the state_dict / checkpoint layout stays the reference's.  nn.DataParallel
+        # replicas share the dict (a shallow copy of __dict__), so every device keeps its state across steps.
+        states = self.__dict__.setdefault("_dropout_rng", {})
+        key = str(eng.device)
+        rng = states.get(key)
+        if rng is None:
+            if torch.cuda.is_current_stream_capturing():
+                raise RuntimeError("the first pass that draws dropout masks on %s is being captured in a CUDA graph: run "
+                                   "it eagerly once first (its random state is created then)" % key)
+            rng = states[key] = DropoutRNG(eng.device)
+        views = eng.dropout_masks(rng, n, [(i, c, float(m.p)) for i, _, m, c in act])
+        rng.last = {name: v[:, :c] for (_, name, _, c), v in zip(act, views)}
+        return {name: v for (_, name, _, _), v in zip(act, views)}
+
+    def dropout_keep(self, device=None):
+        """{Dropout3d module name: float32 [N, C] keep factors} of the last pass that drew masks on ``device`` (default:
+        the parameters' device): 0 for a dropped channel, 1/(1-p) for a kept one.  Views of the pass's own buffer, valid
+        until the next forward; after a replay of a captured step they hold that replay's masks."""
+        if device is None:
+            device = self._weight_tensors()[0].device
+        rng = self.__dict__.get("_dropout_rng", {}).get(str(torch.device(device)))
+        return dict(rng.last) if rng is not None else {}
+
     def _validate(self, x: torch.Tensor):
         if not isinstance(x, torch.Tensor) or x.dim() != 5:
             raise ValueError("expected a 5-D [B, C, D, H, W] tensor")
@@ -213,7 +256,8 @@ def _run_planned(net, eng: Engine, x, record: bool, params, device=None):
         return out
     store = net.__dict__.setdefault("_prep_plans", {})
     key = (tuple(x.shape), str(device if device is not None else x.device), net.compute_dtype, bool(net.training), record,
-           eng.want_input_grad, E.UP_FUSION, E.CONV_PATH, eng.patch_src is not None, eng.label_dst is not None)
+           eng.want_input_grad, E.UP_FUSION, E.CONV_PATH, eng.patch_src is not None, eng.label_dst is not None,
+           net._dropout_config())
     owners = store.setdefault("__owners__", {})
     held = owners.get(key)
     if held is None or len(held) != len(params) or any(a is not b for a, b in zip(held, params)):
@@ -286,7 +330,7 @@ class _GraphNetFn(torch.autograd.Function):
         from . import engine as E
         store = net.__dict__.setdefault("_dropin_graphs", {})
         want_dx = bool(ctx.needs_input_grad[1])
-        key = (tuple(x.shape), str(x.device), net.compute_dtype, want_dx, E.UP_FUSION, E.CONV_PATH)
+        key = (tuple(x.shape), str(x.device), net.compute_dtype, want_dx, E.UP_FUSION, E.CONV_PATH, net._dropout_config())
         st = store.get(key)
         if st is None:
             st = store[key] = _GraphState()
@@ -379,6 +423,7 @@ class UNet(_FusedNet):
         _check_conv_geometry(kern_sz_conv, padding, stride_conv)
         self._k = kern_sz_conv
         self._dropout_p = dropout_p
+        self._dropout_rng = {}        # device -> engine.DropoutRNG (created by the first pass that draws masks there)
 
         self.mp = nn.MaxPool3d(kernel_size=2, padding=0, stride=2, dilation=1, return_indices=True)
         d_blocks, u_blocks = [], []
@@ -407,6 +452,11 @@ class UNet(_FusedNet):
     def _levels(self):
         return len(self.d_blocks)
 
+    def _dropout_sites(self):
+        # (the center block's Dropout3d is not a site: its output is discarded, models.py:238-241, DESIGN.md section 1)
+        return ([("d_blocks.%d.block.6" % i, b.block[6], b.block[4].num_features) for i, b in enumerate(self.d_blocks)]
+                + [("u_blocks.%d.block.7" % i, b.block[7], b.block[5].num_features) for i, b in enumerate(self.u_blocks)])
+
     def _head_flags(self):
         f = 0
         if self.apply_softmax:
@@ -421,12 +471,11 @@ class UNet(_FusedNet):
 
     def _run(self, eng: Engine, x, training):
         """UNet.forward (models.py:226-261) as fused stages."""
-        if training and self._dropout_p:
-            raise NotImplementedError("dropout_p > 0 in training is outside the hot path (every preset uses 0)")
         k = self._k
         extra = 1 if self.chk else 0          # checkpoint recomputation: one more BN buffer update at backward
         cur = eng.pack(x)
         eng.input_act = cur
+        keep = self._draw_dropout(eng, x.shape[0])
         skips = []
         for i, blk in enumerate(self.d_blocks):
             seq = blk.block
@@ -434,7 +483,8 @@ class UNet(_FusedNet):
                          leaf_input=(i == 0))
             a = eng.bn_relu(y, seq[1], training, extra)
             y = eng.conv([a], seq[3].weight, seq[3].bias, k, [True], training)
-            s, cur = eng.bn_relu(y, seq[4], training, extra, pool=True)        # skip tensor + MaxPool (models.py:233)
+            s, cur = eng.bn_relu(y, seq[4], training, extra, pool=True,        # skip tensor + MaxPool (models.py:233)
+                                 keep=keep.get("d_blocks.%d.block.6" % i))
             skips.append(s)
         if training:
             # models.py:238-241 -- the center block runs (its BatchNorm buffers move once) and its output is
@@ -453,7 +503,7 @@ class UNet(_FusedNet):
             y = _up_stage(eng, srcs, seq[0], seq[1], k, training)
             a = eng.bn_relu(y, seq[2], training, extra)
             y = eng.conv([a], seq[4].weight, seq[4].bias, k, [True], training)
-            ubl = eng.bn_relu(y, seq[5], training, extra)
+            ubl = eng.bn_relu(y, seq[5], training, extra, keep=keep.get("u_blocks.%d.block.7" % i))
             srcs = [ubl, skips[-i - 1]] if self.skip else [ubl]                  # models.py:247-253 (cat folded)
         return eng.head(srcs, self.last_conv.weight, self.last_conv.bias, self._head_flags())
 
@@ -541,6 +591,7 @@ class recAE_v2_fixed(_FusedNet):
         _check_conv_geometry(kern_sz_conv, padding)
         self._k = kern_sz_conv
         self._dropout_p = dropout_p
+        self._dropout_rng = {}        # device -> engine.DropoutRNG (created by the first pass that draws masks there)
         fms = [i_size * pow(2, n) for n in range(5)]
         self.mp = nn.MaxPool3d(kernel_size=2, padding=0, stride=2, dilation=1, return_indices=True)
         self.dblock1 = down_block_cr(input_channels, fms[0], kern_s=kern_sz_conv, pad=padding, dropout_p=dropout_p)
@@ -563,33 +614,39 @@ class recAE_v2_fixed(_FusedNet):
     def _levels(self):
         return 4
 
+    def _dropout_sites(self):
+        downs = [("dblock%d.6" % n, m[6], m[4].num_features)
+                 for n, m in enumerate([self.dblock1, self.dblock2, self.dblock3, self.dblock4], 1)]
+        ups = [("ublock%d.7" % n, m[7], m[5].num_features)
+               for n, m in enumerate([self.ublock1, self.ublock2, self.ublock3, self.ublock4], 1)]
+        return downs + [("cblock_center.6", self.cblock_center[6], self.cblock_center[4].num_features)] + ups
+
     def _run(self, eng: Engine, x, training):
         """recAE_v2_fixed.forward (models.py:509-538)."""
-        if training and self._dropout_p:
-            raise NotImplementedError("dropout_p > 0 in training is outside the hot path (every preset uses 0)")
         k = self._k
         extra = 1 if self.chk else 0
         cur = eng.pack(x)
         eng.input_act = cur
+        keep = self._draw_dropout(eng, x.shape[0])
         skips = []
         for i, seq in enumerate([self.dblock1, self.dblock2, self.dblock3, self.dblock4]):
             y = eng.conv([cur], seq[0].weight, seq[0].bias, k, [eng.want_input_grad if i == 0 else True], training,
                          leaf_input=(i == 0))
             a = eng.bn_relu(y, seq[1], training, extra)
             y = eng.conv([a], seq[3].weight, seq[3].bias, k, [True], training)
-            s, cur = eng.bn_relu(y, seq[4], training, extra, pool=True)
+            s, cur = eng.bn_relu(y, seq[4], training, extra, pool=True, keep=keep.get("dblock%d.6" % (i + 1)))
             skips.append(s)
         seq = self.cblock_center
         y = eng.conv([cur], seq[0].weight, seq[0].bias, k, [True], training)
         a = eng.bn_relu(y, seq[1], training, extra)
         y = eng.conv([a], seq[3].weight, seq[3].bias, k, [True], training)
-        cur = eng.bn_relu(y, seq[4], training, extra)
+        cur = eng.bn_relu(y, seq[4], training, extra, keep=keep.get("cblock_center.6"))
         srcs = [cur]
         for i, seq in enumerate([self.ublock1, self.ublock2, self.ublock3, self.ublock4]):
             y = _up_stage(eng, srcs, seq[0], seq[1], k, training)
             a = eng.bn_relu(y, seq[2], training, extra)
             y = eng.conv([a], seq[4].weight, seq[4].bias, k, [True], training)
-            up = eng.bn_relu(y, seq[5], training, extra)
+            up = eng.bn_relu(y, seq[5], training, extra, keep=keep.get("ublock%d.7" % (i + 1)))
             srcs = [up, skips[3 - i]]                                            # models.py:528-534
         return eng.head(srcs, self.last_conv.weight, self.last_conv.bias, _lib.HEAD_SOFTMAX)   # models.py:538
 

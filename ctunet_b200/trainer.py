@@ -99,6 +99,11 @@ class _LossSpec:
         return [r[1] for r in res], [r[0] for r in res]
 
 
+def _dropout_ps(model):
+    """p of every Dropout3d site (a training step puts them all in train mode): what a captured step's masks depend on."""
+    return tuple(float(m.p) for _, m, _ in model._dropout_sites())
+
+
 class TrainStep:
     """``step(image, target)`` enqueues one full training iteration and returns the device tensor
     ``[components..., total]`` in the order of ``keys`` (no host sync).  In graph mode the returned tensor is the graph's
@@ -141,6 +146,7 @@ class TrainStep:
         self._static = None
         self._static_out = None
         self._calls = 0
+        self._dropout_cfg = None                              # Dropout3d sites / p the captured step draws masks for
         self.launches_per_step = None                         # C-ABI calls recorded in the captured step
 
     # ------------------------------------------------------------------ one iteration, enqueued on the current stream
@@ -195,6 +201,8 @@ class TrainStep:
             self._static = [torch.empty_like(t) for t in flat]
         elif any(a.shape != b.shape or a.dtype != b.dtype for a, b in zip(flat, self._static)):
             raise RuntimeError("graph mode: the batch shape changed after the step was captured")
+        elif _dropout_ps(self.model) != self._dropout_cfg:
+            raise RuntimeError("graph mode: the Dropout3d configuration (p of a site) changed after the step was captured")
         for dst, src in zip(self._static, flat):
             if dst.data_ptr() != src.data_ptr():              # a pipeline may fill static_inputs() in place
                 dst.copy_(src, non_blocking=True)
@@ -222,6 +230,7 @@ class TrainStep:
                     self._update(self._static_out)
                 self._graph_opt = g2
             self.launches_per_step = _lib.launches - l0
+            self._dropout_cfg = _dropout_ps(self.model)
             self._graph = g
         return self._replay()
 

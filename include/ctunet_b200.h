@@ -44,6 +44,7 @@ extern "C" {
  * the caller has already zeroed the double accumulators (bn_sums / sums / sums2), so the entry point enqueues no memset of
  * its own.  A step driver zeroes ONE arena for all of a pass's accumulators instead of ~30 memset nodes on the layer chain. */
 #define CTU_ACCUM_PREZEROED 0x100
+#define CTU_DROPOUT_MAX_SITES 32
 
 typedef enum { CTU_F32 = 0, CTU_BF16 = 1 } ctu_dtype;
 typedef void* ctu_stream; /* cudaStream_t */
@@ -186,6 +187,28 @@ int ctu_bn_relu_fwd_train(int dtype, const void* y, const double* sums, double c
                           float* running_mean, float* running_var, long long* num_batches_tracked, float momentum, float eps,
                           int n_updates, float* ss, void* a, void* pooled, int c, int n, int d, int h, int w,
                           int y_phase_major, ctu_stream stream);
+/* _drop variants: keep (nullable, float[n][cpad]) = the Dropout3d keep factors k[n][c] of the site that follows the ReLU
+ * (ctu_dropout3d_keep): a = round(k * relu(scale*y + shift)) and pooled = maxpool2 of those values.  The backward variants
+ * take the same factors: dz = k * (dA + unpool(dP)) * [scale*y + shift > 0].  NULL = the plain entry points above / below.
+ * A phase-major y never precedes a dropout site and is refused with keep != NULL. */
+int ctu_bn_relu_fwd_drop(int dtype, const void* y, const float* ss, void* a, void* pooled, int c, int n, int d, int h,
+                         int w, int y_phase_major, const float* keep, ctu_stream stream);
+int ctu_bn_relu_fwd_train_drop(int dtype, const void* y, const double* sums, double count, const float* gamma,
+                               const float* beta, float* running_mean, float* running_var, long long* num_batches_tracked,
+                               float momentum, float eps, int n_updates, float* ss, void* a, void* pooled, int c, int n,
+                               int d, int h, int w, int y_phase_major, const float* keep, ctu_stream stream);
+int ctu_bn_relu_bwd_reduce_drop(int dtype, const void* y, const float* ss, const void* dA, const void* dP, double* sums2,
+                                int c, int n, int d, int h, int w, int y_phase_major, const float* keep, ctu_stream stream);
+int ctu_bn_relu_bwd_apply_drop(int dtype, const void* y, const float* ss, const float* gamma, const void* dA, const void* dP,
+                               const double* sums2, double count, void* dy, float* dgamma, float* dbeta, int c, int n, int d,
+                               int h, int w, int y_phase_major, const float* keep, ctu_stream stream);
+/* Dropout3d keep factors of the nsite sites of one pass (nsite <= CTU_DROPOUT_MAX_SITES), site i at
+ * keep + n * (cpad_0 + ... + cpad_{i-1}) as float[n][cpad_i], cpad_i = 8*ceil(h_channels[i]/8):
+ * k = 1/(1-p) with probability 1-p, else 0 (p = 1: all zero; pad lanes 0).  Philox4x32-10 keyed by `seed`, counter =
+ * (pass, h_site[i], sample*cpad_i + channel) with pass = *pass_counter, which the launch then advances by one (so a replayed
+ * CUDA graph draws new masks every replay); pass_counter NULL: pass 0, nothing advanced.  One block, no host sync. */
+int ctu_dropout3d_keep(int nsite, const int* h_site, const int* h_channels, const float* h_p, int n,
+                       unsigned long long seed, unsigned long long* pass_counter, float* keep, ctu_stream stream);
 /* backward, pass 1: sums2 = double[2*cpad] = sum(dz), sum(dz*xhat) with
  * dz = (dA + unpool(dP)) * [a > 0]; dA and dP are nullable (not both) */
 int ctu_bn_relu_bwd_reduce(int dtype, const void* y, const float* ss, const void* dA, const void* dP, double* sums2,
