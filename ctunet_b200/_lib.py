@@ -36,6 +36,8 @@ SIGNATURES = {
     "ctu_unpack_ncdhw": (I, [P, P, I, I, I, LL, P]),
     "ctu_pack_patches": (I, [P, P, P, I, I, I, I, I, I, I, P]),
     "ctu_head_labels": (I, [I, P, P, I, P, P, I, I, P, I, I, I, I, P, P, I, LL, P]),
+    "ctu_head_accumulate": (I, [I, P, P, I, P, P, I, I, P, I, I, I, I, P, P, I, LL, P]),
+    "ctu_window_finalize": (I, [P, I, I, I, I, I, P, P, P, P, P, P]),
     "ctu_conv_wpack_floats": (LL, [I, I, I, P]),
     "ctu_conv_pack_weight": (I, [P, P, I, I, I, P, P]),
     "ctu_conv_wpack_dgrad_floats": (LL, [I, I, I]),

@@ -898,6 +898,146 @@ static int head_labels_launch(const HeadParams& p, const int* origins, int patch
     return check_launch("ctu_head_labels");
 }
 
+// ------------------------------------------------------------------------------------------------ head -> blended sums
+// Overlapping sliding-window inference (preprocess.sliding_window_predict, DESIGN.md section 7b).  Every window voxel
+// inside the [vd][vh][vw] volume adds, for each head output channel v (the values ctu_head_fwd writes, all in [0, 2] for
+// a head with softmax / sigmoid), llrint(w * v * 2^40) to acc[out][c][z][y][x], with the separable window weight
+// w = wt[z] * wt[p + y] * wt[2p + x] (fp32).  Integer sums do not depend on the order of the additions: the blended
+// result is bit-identical whatever the batch, the window order or the number of ranks.  The return values of the 64-bit
+// atomics are unused, so they compile to reductions (RED.E.ADD.64).
+constexpr float kAccScale = 1099511627776.f;      // 2^40
+
+__device__ __forceinline__ void acc_add(long long* a, float v) {
+    atomicAdd(reinterpret_cast<unsigned long long*>(a), (unsigned long long)__float2ll_rn(v * kAccScale));
+}
+
+template <typename T, int CO, int CBT>
+__global__ void __launch_bounds__(kHeadThreads) head_accum_kernel(HeadParams p, const int* __restrict__ origins, int patch,
+                                                                  int vd, int vh, int vw, const float* __restrict__ wt,
+                                                                  long long* __restrict__ acc) {
+    extern __shared__ float hsm[];
+    float* wsm = hsm;
+    float* bsm = hsm + CO * CBT * 8;
+    load_head_weights<CO>(p, wsm, bsm);
+    __syncthreads();
+    const long long total = (long long)p.n * p.spatial;
+    const long long plane = (long long)vd * vh * vw;
+    const bool sp = (p.flags & (CTU_HEAD_SP | CTU_HEAD_SP_SOFTMAX)) != 0;
+    for (long long i = (long long)blockIdx.x * kHeadThreads + threadIdx.x; i < total; i += (long long)gridDim.x * kHeadThreads) {
+        const int n = (int)(i / p.spatial);
+        const long long s = i % p.spatial;
+        const int x = (int)(s % patch), y = (int)((s / patch) % patch), z = (int)(s / ((long long)patch * patch));
+        const int gz = origins[3 * n] + z, gy = origins[3 * n + 1] + y, gx = origins[3 * n + 2] + x;
+        if (gz < 0 || gz >= vd || gy < 0 || gy >= vh || gx < 0 || gx >= vw) continue;   // outputs past the volume: dropped
+        HeadVals<CO> h;
+        V8 xs[CBT];
+        head_logits<T, CO, CBT>(p, wsm, bsm, n, s, h, xs);
+        head_forward_chain<CO>(h, p.flags);
+        const float w = __ldg(wt + z) * __ldg(wt + patch + y) * __ldg(wt + 2 * patch + x);
+        long long* a = acc + ((long long)gz * vh + gy) * vw + gx;
+        if (sp) {
+            acc_add(a, w * h.o0[0]);
+            acc_add(a + plane, w * h.o0[1]);
+            acc_add(a + 2 * plane, w * h.o1[0]);
+            acc_add(a + 3 * plane, w * h.o1[1]);
+        } else {
+#pragma unroll
+            for (int c = 0; c < CO; ++c) acc_add(a + c * plane, w * h.sg[c]);
+        }
+    }
+}
+
+template <typename T, int CO>
+static int head_accum_launch(const HeadParams& p, const int* origins, int patch, int vd, int vh, int vw, const float* wt,
+                             long long* acc, cudaStream_t stream) {
+    const size_t smem = (size_t)(CO * p.m.cb_total * 8 + 8) * sizeof(float);
+    const long long total = (long long)p.n * p.spatial;
+    const int grid = (int)((total + kHeadThreads - 1) / kHeadThreads > 148 * 32 ? 148 * 32 : (total + kHeadThreads - 1) / kHeadThreads);
+    switch (p.m.cb_total) {
+        case 1: head_accum_kernel<T, CO, 1><<<grid, kHeadThreads, smem, stream>>>(p, origins, patch, vd, vh, vw, wt, acc); break;
+        case 2: head_accum_kernel<T, CO, 2><<<grid, kHeadThreads, smem, stream>>>(p, origins, patch, vd, vh, vw, wt, acc); break;
+        case 3: head_accum_kernel<T, CO, 3><<<grid, kHeadThreads, smem, stream>>>(p, origins, patch, vd, vh, vw, wt, acc); break;
+        default: head_accum_kernel<T, CO, 4><<<grid, kHeadThreads, smem, stream>>>(p, origins, patch, vd, vh, vw, wt, acc); break;
+    }
+    return check_launch("ctu_head_accumulate");
+}
+
+// Finalize of the blended sums: labels[o] = argmax over the C channels of acc[o] (first maximum wins; the per-voxel
+// normaliser is a positive common factor, so the integer sums decide) and, when probs[o] is given, the blended values
+// acc * 2^-40 / (nz[z] * ny[y] * nx[x]) from the float64 per-axis normaliser tables norm = [nz | ny | nx].
+// One pass over the accumulators; VEC: four voxels per thread, 16-byte loads and stores (the plane size is a multiple
+// of 4 and the buffers are 16-byte aligned).
+template <int C, bool VEC>
+__global__ void window_finalize_kernel(const long long* __restrict__ acc, int n_out, int vd, int vh, int vw,
+                                       const double* __restrict__ norm, float* l0, float* l1, float* q0, float* q1) {
+    const long long plane = (long long)vd * vh * vw;
+    const long long nitem = VEC ? plane >> 2 : plane;
+    constexpr int V = VEC ? 4 : 1;
+    for (long long it = (long long)blockIdx.x * blockDim.x + threadIdx.x; it < nitem; it += (long long)gridDim.x * blockDim.x) {
+        const long long v0 = it * V;
+        double r[V];
+        if (q0 != nullptr) {
+#pragma unroll
+            for (int k = 0; k < V; ++k) {
+                const long long v = v0 + k;
+                const int x = (int)(v % vw), y = (int)((v / vw) % vh), z = (int)(v / ((long long)vw * vh));
+                r[k] = 0x1p-40 / (norm[z] * norm[vd + y] * norm[vd + vh + x]);
+            }
+        }
+        for (int o = 0; o < n_out; ++o) {
+            long long a[C][V];
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                const long long* src = acc + ((long long)o * C + c) * plane + v0;
+                if constexpr (VEC) {
+                    const longlong2 u = __ldg(reinterpret_cast<const longlong2*>(src));
+                    const longlong2 w = __ldg(reinterpret_cast<const longlong2*>(src) + 1);
+                    a[c][0] = u.x; a[c][1] = u.y; a[c][2] = w.x; a[c][3] = w.y;
+                } else {
+                    a[c][0] = __ldg(src);
+                }
+            }
+            float lab[V];
+#pragma unroll
+            for (int k = 0; k < V; ++k) {
+                int bi = 0;
+#pragma unroll
+                for (int c = 1; c < C; ++c)
+                    if (a[c][k] > a[bi][k]) bi = c;
+                lab[k] = (float)bi;
+            }
+            float* lo = o == 0 ? l0 : l1;
+            if constexpr (VEC) *reinterpret_cast<float4*>(lo + v0) = make_float4(lab[0], lab[1], lab[2], lab[3]);
+            else lo[v0] = lab[0];
+            float* qo = o == 0 ? q0 : q1;
+            if (qo == nullptr) continue;
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                float f[V];
+#pragma unroll
+                for (int k = 0; k < V; ++k) f[k] = (float)((double)a[c][k] * r[k]);
+                float* dst = qo + (long long)c * plane + v0;
+                if constexpr (VEC) *reinterpret_cast<float4*>(dst) = make_float4(f[0], f[1], f[2], f[3]);
+                else dst[0] = f[0];
+            }
+        }
+    }
+}
+
+template <int C>
+static int window_finalize_launch(const long long* acc, int n_out, int vd, int vh, int vw, const double* norm, float* l0,
+                                  float* l1, float* q0, float* q1, cudaStream_t stream) {
+    const long long plane = (long long)vd * vh * vw;
+    bool vec = plane % 4 == 0;
+    for (const void* ptr : {(const void*)acc, (const void*)l0, (const void*)l1, (const void*)q0, (const void*)q1})
+        vec = vec && (reinterpret_cast<uintptr_t>(ptr) & 15u) == 0;
+    const long long items = vec ? plane / 4 : plane;
+    const int grid = (int)((items + 255) / 256 > 148 * 16 ? 148 * 16 : (items + 255) / 256);
+    if (vec) window_finalize_kernel<C, true><<<grid, 256, 0, stream>>>(acc, n_out, vd, vh, vw, norm, l0, l1, q0, q1);
+    else window_finalize_kernel<C, false><<<grid, 256, 0, stream>>>(acc, n_out, vd, vh, vw, norm, l0, l1, q0, q1);
+    return check_launch("ctu_window_finalize");
+}
+
 }  // namespace ctu
 
 using namespace ctu;
@@ -1070,6 +1210,44 @@ int ctu_head_labels(int dtype, const void* const* h_srcs, const int* h_src_chann
         }
     });
     return CTU_OK;
+}
+
+int ctu_head_accumulate(int dtype, const void* const* h_srcs, const int* h_src_channels, int nsrc, const float* w,
+                        const float* bias, int cout, int flags, const int* origins, int patch, int vd, int vh, int vw,
+                        const float* weights, long long* acc, int n, long long spatial, ctu_stream stream) {
+    HeadParams p = {};
+    int rc = head_setup(p, h_srcs, h_src_channels, nsrc, w, bias, cout, flags, n, spatial, "ctu_head_accumulate");
+    if (rc != CTU_OK) return rc;
+    CTU_REQUIRE(origins && weights && acc, "ctu_head_accumulate: missing origins / weights / accumulators");
+    CTU_REQUIRE(patch > 0 && (long long)patch * patch * patch == spatial && vd > 0 && vh > 0 && vw > 0,
+                "ctu_head_accumulate: needs spatial = patch^3 and a non-empty volume");
+    CTU_REQUIRE(flags & (CTU_HEAD_SOFTMAX | CTU_HEAD_SIGMOID | CTU_HEAD_SP_SOFTMAX),
+                "ctu_head_accumulate: the head outputs must be bounded (softmax or sigmoid) for the fixed-point sums");
+    CTU_DISPATCH_DTYPE(dtype, {
+        switch (cout) {
+            case 1: return head_accum_launch<T, 1>(p, origins, patch, vd, vh, vw, weights, acc, (cudaStream_t)stream);
+            case 2: return head_accum_launch<T, 2>(p, origins, patch, vd, vh, vw, weights, acc, (cudaStream_t)stream);
+            case 3: return head_accum_launch<T, 3>(p, origins, patch, vd, vh, vw, weights, acc, (cudaStream_t)stream);
+            default: return head_accum_launch<T, 4>(p, origins, patch, vd, vh, vw, weights, acc, (cudaStream_t)stream);
+        }
+    });
+    return CTU_OK;
+}
+
+int ctu_window_finalize(const long long* acc, int n_out, int channels, int vd, int vh, int vw, const double* norm,
+                        float* labels0, float* labels1, float* probs0, float* probs1, ctu_stream stream) {
+    CTU_REQUIRE(acc && labels0 && vd > 0 && vh > 0 && vw > 0 && (n_out == 1 || (n_out == 2 && labels1)),
+                "ctu_window_finalize: bad arguments (n_out 1 or 2, one label volume per output)");
+    CTU_REQUIRE(channels >= 1 && channels <= 4, "ctu_window_finalize: channels must be 1..4");
+    CTU_REQUIRE(!probs0 || (norm && (n_out == 1 || probs1)), "ctu_window_finalize: probabilities need the normaliser "
+                "tables and one output per head output");
+    const cudaStream_t st = (cudaStream_t)stream;
+    switch (channels) {
+        case 1: return window_finalize_launch<1>(acc, n_out, vd, vh, vw, norm, labels0, labels1, probs0, probs1, st);
+        case 2: return window_finalize_launch<2>(acc, n_out, vd, vh, vw, norm, labels0, labels1, probs0, probs1, st);
+        case 3: return window_finalize_launch<3>(acc, n_out, vd, vh, vw, norm, labels0, labels1, probs0, probs1, st);
+        default: return window_finalize_launch<4>(acc, n_out, vd, vh, vw, norm, labels0, labels1, probs0, probs1, st);
+    }
 }
 
 }  // extern "C"

@@ -76,9 +76,13 @@ __global__ void pack4_kernel(const float* __restrict__ src, T* __restrict__ dst,
 
 // Patch gather for sliding-window inference: B patches of p^3 voxels out of a float32 [C][D][H][W] volume at the origins
 // listed in device memory -> blocked [B][Cb][p][p][p][8].  Four x-consecutive voxels per thread (16-byte loads per channel).
+// A patch that lies inside the volume with a 16-byte aligned x origin (vec4: the volume width is a multiple of 4 and the
+// volume is 16-byte aligned) takes the float4 loads; any other window -- an origin anywhere, a width that is not a
+// multiple of 4, a window reaching past a face -- reads voxel by voxel and zero-fills whatever lies outside the volume.
+// The origins are device data, so the choice is made per patch here.
 template <typename T>
 __global__ void pack_patches_kernel(const float* __restrict__ vol, const int* __restrict__ origins, T* __restrict__ dst, int c,
-                                    int cb, int D, int H, int W, int p, long long total4) {
+                                    int cb, int D, int H, int W, int p, long long total4, int vec4) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total4) return;
     const int p4 = p >> 2;
@@ -90,12 +94,28 @@ __global__ void pack_patches_kernel(const float* __restrict__ vol, const int* __
     const int n = (int)(r / cb);
     const int oz = origins[3 * n], oy = origins[3 * n + 1], ox = origins[3 * n + 2];
     const long long plane = (long long)D * H * W;
-    const long long src0 = ((long long)(oz + z) * H + (oy + y)) * W + ox + 4 * x4;
     float4 v[8];
+    const bool inside = oz >= 0 && oy >= 0 && ox >= 0 && oz + p <= D && oy + p <= H && ox + p <= W;
+    if (vec4 && inside && (ox & 3) == 0) {
+        const long long src0 = ((long long)(oz + z) * H + (oy + y)) * W + ox + 4 * x4;
 #pragma unroll
-    for (int j = 0; j < 8; ++j) {
-        const int ch = b * 8 + j;
-        v[j] = ch < c ? __ldg(reinterpret_cast<const float4*>(vol + ch * plane + src0)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int j = 0; j < 8; ++j) {
+            const int ch = b * 8 + j;
+            v[j] = ch < c ? __ldg(reinterpret_cast<const float4*>(vol + ch * plane + src0)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+    } else {
+        const int gz = oz + z, gy = oy + y, gx = ox + 4 * x4;
+        const bool row = gz >= 0 && gz < D && gy >= 0 && gy < H;
+        const long long src0 = ((long long)gz * H + gy) * W + gx;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const int ch = b * 8 + j;
+            float e[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+                e[k] = (ch < c && row && gx + k >= 0 && gx + k < W) ? __ldg(vol + ch * plane + src0 + k) : 0.f;
+            v[j] = make_float4(e[0], e[1], e[2], e[3]);
+        }
     }
     T* out = dst + (((((long long)n * cb + b) * p + z) * p + y) * p + 4 * x4) * 8;
     V8 q;
@@ -248,11 +268,12 @@ int ctu_pack_ncdhw(const float* src, void* dst, int dtype, int n, int c, long lo
 int ctu_pack_patches(const float* vol, const int* origins, void* dst, int dtype, int n, int c, int vd, int vh, int vw, int patch,
                      ctu_stream stream) {
     CTU_REQUIRE(vol && origins && dst && n > 0 && c > 0 && vd > 0 && vh > 0 && vw > 0, "ctu_pack_patches: bad arguments");
-    CTU_REQUIRE(patch > 0 && patch % 4 == 0 && vw % 4 == 0, "ctu_pack_patches: patch size and volume width must be multiples of 4");
+    CTU_REQUIRE(patch > 0 && patch % 4 == 0, "ctu_pack_patches: the patch size must be a multiple of 4");
     const int cb = (c + 7) / 8;
     const long long total4 = (long long)n * cb * patch * patch * (patch / 4);
+    const int vec4 = vw % 4 == 0 && (reinterpret_cast<uintptr_t>(vol) & 15u) == 0;
     CTU_DISPATCH_DTYPE(dtype, (pack_patches_kernel<T><<<cdiv(total4, 256), 256, 0, (cudaStream_t)stream>>>(
-                                  vol, origins, (T*)dst, c, cb, vd, vh, vw, patch, total4)));
+                                  vol, origins, (T*)dst, c, cb, vd, vh, vw, patch, total4, vec4)));
     return check_launch("ctu_pack_patches");
 }
 

@@ -197,6 +197,9 @@ class Engine:
         # gather, (labels, origins, patch, dims) makes the head write hard labels (scattered at the origins when given)
         self.patch_src = None
         self.label_dst = None
+        # overlapping windows (models._FusedNet.accumulate_windows): (acc, origins, patch, dims, weight table) makes the
+        # head add its weighted outputs to the int64 accumulators instead (csrc/head.cu: head_accum_kernel)
+        self.accum_dst = None
         self._keep_event = None                    # Dropout3d keep factors drawn on their own stream (see dropout_masks)
 
     # ------------------------------------------------------------------ weight preparation on a side stream
@@ -1004,6 +1007,14 @@ class Engine:
             call("ctu_head_labels", self.dtype, pa, ca, ns, weight.data_ptr(), bias.data_ptr(), cout, flags,
                  origins.data_ptr() if origins is not None else None, int(patch), vd, vh, vw, labels[0].data_ptr(),
                  labels[1].data_ptr() if sp else None, s0.n, s0.spatial, stream_ptr())
+            return None
+        if self.accum_dst is not None:
+            acc, origins, patch, dims, wtab = self.accum_dst
+            nch = 4 if sp else cout
+            if acc.dtype != torch.int64 or acc.numel() != nch * dims[0] * dims[1] * dims[2]:
+                raise ValueError("the %s head accumulates into int64 [%d, D, H, W]" % ("SP" if sp else "plain", nch))
+            call("ctu_head_accumulate", self.dtype, pa, ca, ns, weight.data_ptr(), bias.data_ptr(), cout, flags,
+                 origins.data_ptr(), int(patch), *dims, wtab.data_ptr(), acc.data_ptr(), s0.n, s0.spatial, stream_ptr())
             return None
         if self.fused_loss is not None:
             return self._head_loss(list(srcs), weight, bias, flags, sp)

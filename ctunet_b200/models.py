@@ -242,6 +242,36 @@ class _FusedNet(nn.Module):
         finally:
             self.train(was)
 
+    @torch.no_grad()
+    def accumulate_windows(self, *, vol, origins, patch, weights, acc):
+        """Overlapping sliding-window mode (preprocess.sliding_window_predict): eval-mode forward of the B windows of
+        ``patch``^3 voxels at the device int32 ``origins`` [B,3] (z, y, x; anywhere: input voxels outside ``vol`` read as 0),
+        gathered from ``vol`` float32 [C,D,H,W], and every window voxel inside the volume adds its weighted head outputs to
+        the int64 accumulators ``acc`` [n_out * channels, D, H, W] in 2^-40 fixed point.  ``weights`` is the device
+        float32 [3, patch] table of the separable window weight.  Returns ``acc``."""
+        was = self.training
+        self.eval()
+        try:
+            if not (vol.is_cuda and vol.dtype == torch.float32 and vol.dim() == 4 and vol.is_contiguous()):
+                raise TypeError("vol: contiguous float32 CUDA tensor [C, D, H, W]")
+            if not (origins.is_cuda and origins.dtype == torch.int32 and origins.dim() == 2 and origins.shape[1] == 3):
+                raise TypeError("origins: CUDA int32 tensor [B, 3]")
+            if not (weights.is_cuda and weights.dtype == torch.float32 and tuple(weights.shape) == (3, patch)):
+                raise TypeError("weights: CUDA float32 tensor [3, patch]")
+            if not (acc.is_cuda and acc.dtype == torch.int64 and acc.is_contiguous() and acc.shape[1:] == vol.shape[1:]):
+                raise TypeError("acc: contiguous int64 CUDA tensor [n_out * channels, D, H, W]")
+            m = 2 ** self._levels()
+            if patch % m or patch % 4:
+                raise ValueError("patch size %d must be divisible by %d" % (patch, max(m, 4)))
+            eng = Engine(vol.device, self.compute_dtype, record=False)
+            eng.patch_src = (vol, origins.contiguous(), int(patch))
+            eng.accum_dst = (acc, origins.contiguous(), int(patch), tuple(vol.shape[1:]), weights.contiguous())
+            shape = torch.empty((origins.shape[0], vol.shape[0], patch, patch, patch), device="meta")
+            _run_planned(self, eng, shape, False, params=self._weight_tensors(), device=vol.device)
+            return acc
+        finally:
+            self.train(was)
+
 
 def _run_planned(net, eng: Engine, x, record: bool, params, device=None):
     """Run the network with the weight-preparation plan of this (shape, mode) configuration (Engine.begin).
@@ -257,7 +287,7 @@ def _run_planned(net, eng: Engine, x, record: bool, params, device=None):
     store = net.__dict__.setdefault("_prep_plans", {})
     key = (tuple(x.shape), str(device if device is not None else x.device), net.compute_dtype, bool(net.training), record,
            eng.want_input_grad, E.UP_FUSION, E.CONV_PATH, eng.patch_src is not None, eng.label_dst is not None,
-           net._dropout_config())
+           net._dropout_config(), eng.accum_dst is not None)
     owners = store.setdefault("__owners__", {})
     held = owners.get(key)
     if held is None or len(held) != len(params) or any(a is not b for a, b in zip(held, params)):

@@ -8,6 +8,9 @@ patch grid) -- parity with the reference is therefore unpinned by construction.
 """
 from __future__ import annotations
 
+import math
+
+import numpy as np
 import torch
 
 from ._lib import call, stream_ptr
@@ -99,24 +102,39 @@ def _captured_patch_labels(model, xb: torch.Tensor):
     return outs
 
 
-def _captured_fused_pass(model, vol, patch, batch, n_out):
-    """(static volume, static label volumes, static origins [batch, 3], graph) of one fused patch-batch pass
-    (gather -> network -> labels scattered at the origins), captured once per (model weights, volume shape, patch, batch)."""
+def _captured_fused_pass(model, vol, patch, batch, n_out, accum=None):
+    """(static volume, static outputs, static origins [batch, 3], graph) of one fused patch-batch pass, captured once per
+    (model weights, volume shape, patch, batch, pass kind).  ``accum`` None: gather -> network -> labels scattered at the
+    origins; the static outputs are the label volumes.  ``accum`` = (blend, sigma_scale, channels): gather -> network ->
+    weighted head outputs added to the accumulators (``model.accumulate_windows``); the static outputs are
+    [int64 accumulators [channels, D, H, W], float32 weight table [3, patch]]."""
     graphs = model.__dict__.setdefault("_infer_graphs", {})
-    key = ("fused", tuple(vol.shape), str(vol.device), int(patch), int(batch), getattr(model, "compute_dtype", None))
+    kind = "fused" if accum is None else ("accumulate", accum[0], float(accum[1]))
+    key = (kind, tuple(vol.shape), str(vol.device), int(patch), int(batch), getattr(model, "compute_dtype", None))
     weights = list(model.parameters()) + list(model.buffers())
     ent = graphs.get(key)
     if ent is not None and (len(ent[4]) != len(weights) or any(a is not b for a, b in zip(ent[4], weights))):
         ent = None
     if ent is None:
         st_vol = vol.clone()
-        st_outs = [torch.zeros(tuple(vol.shape[1:]), dtype=torch.float32, device=vol.device) for _ in range(n_out)]
         st_org = torch.zeros((batch, 3), dtype=torch.int32, device=vol.device)
-        model.predict_labels(vol=st_vol, origins=st_org, patch=patch, out=st_outs)      # warm-up: plans, allocator pools
+        if accum is None:
+            st_outs = [torch.zeros(tuple(vol.shape[1:]), dtype=torch.float32, device=vol.device) for _ in range(n_out)]
+
+            def run():
+                model.predict_labels(vol=st_vol, origins=st_org, patch=patch, out=st_outs)
+        else:
+            wt = torch.tensor(window_weights(patch, accum[0], accum[1]), dtype=torch.float32)
+            st_outs = [torch.zeros((accum[2],) + tuple(vol.shape[1:]), dtype=torch.int64, device=vol.device),
+                       wt.expand(3, patch).contiguous().to(vol.device)]
+
+            def run():
+                model.accumulate_windows(vol=st_vol, origins=st_org, patch=patch, weights=st_outs[1], acc=st_outs[0])
+        run()                                   # warm-up: plans, allocator pools
         torch.cuda.synchronize()
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g):
-            model.predict_labels(vol=st_vol, origins=st_org, patch=patch, out=st_outs)
+            run()
         ent = (st_vol, st_outs, st_org, g, weights)
         graphs[key] = ent
         if len(graphs) > 8:
@@ -199,3 +217,163 @@ def sliding_window_argmax(model, vol: torch.Tensor, patch: int = 128, batch: int
             dist.all_reduce(o, op=dist.ReduceOp.SUM, group=group)     # disjoint supports: the sum IS the stitch
     model.train(was_training)
     return outs
+
+
+# ------------------------------------------------------------------------------------------------ overlapping windows
+# Semantics (DESIGN.md section 7b; frozen by tests/window_oracle.py -- the reference has no sliding-window code):
+#   grid     per axis of size S, patch p, overlap in [0, 1): step = max(1, floor(p (1 - overlap))); one origin 0 when S <= p
+#            (the window reaches past the volume: its inputs there read as 0, its outputs there are dropped), otherwise
+#            ceil((S - p) / step) + 1 origins min(i step, S - p); the windows are the z-major product of the axis lists.
+#   weights  separable w(z, y, x) = wz[z] wy[y] wx[x]; "constant": 1; "gaussian": max(g(t) / max g, 2^-6) with
+#            g(t) = exp(-(t - (p - 1) / 2)^2 / (2 sigma^2)), sigma = sigma_scale p.
+#   sums     every window voxel inside the volume adds llrint(w v 2^40) to an int64 accumulator per head output channel
+#            value v (in [0, 2]): exact integer sums, independent of batch, window order and ranks.
+#   outputs  labels = argmax over the accumulators (first maximum wins); probabilities = acc 2^-40 / (Nz[z] Ny[y] Nx[x]),
+#            Na[t] = sum of wa[t - o] over the axis origins o whose window covers t.
+ACC_FRACTION_BITS = 40
+_BLENDS = ("constant", "gaussian")
+
+
+def window_origins(size: int, patch: int, overlap: float):
+    """Window origins along one axis of ``size`` voxels (see the grid rule above)."""
+    step = max(1, int(math.floor(patch * (1.0 - overlap))))
+    if size <= patch:
+        return [0]
+    n = -(-(size - patch) // step) + 1
+    return [min(i * step, size - patch) for i in range(n)]
+
+
+def window_weights(patch: int, blend: str = "gaussian", sigma_scale: float = 0.125):
+    """float64 [patch] weight table of one axis.  The 2^-6 floor keeps the 3-D weight >= 2^-18, so a voxel's total
+    weight stays far above the 2^-40 fixed-point resolution of the accumulators."""
+    if blend == "constant":
+        return np.ones(patch, dtype=np.float64)
+    if blend != "gaussian":
+        raise ValueError("blend must be one of %s, got %r" % (_BLENDS, blend))
+    sigma = sigma_scale * patch
+    t = np.arange(patch, dtype=np.float64)
+    g = np.exp(-((t - (patch - 1) / 2.0) ** 2) / (2.0 * sigma * sigma))
+    return np.maximum(g / g.max(), 2.0 ** -6)
+
+
+def window_normaliser(size: int, patch: int, origins, weights):
+    """float64 [size] total weight Na[t] of one axis: the sum of weights[t - o] over the origins o whose window covers t."""
+    n = np.zeros(size, dtype=np.float64)
+    for o in origins:
+        hi = min(o + patch, size)
+        n[o:hi] += np.asarray(weights, dtype=np.float64)[:hi - o]
+    return n
+
+
+def window_grid(shape, patch: int, overlap: float):
+    """Per-axis origin lists of a [D, H, W] volume.  Raises OverflowError when the most-covered voxel could overflow the
+    int64 accumulators: each window adds at most 2 * 2^40 (weight <= 1, head output <= 2)."""
+    axes = [window_origins(int(s), patch, overlap) for s in shape]
+    coverage = 1
+    for s, org in zip(shape, axes):
+        cover = np.zeros(int(s), dtype=np.int64)
+        for o in org:
+            cover[o:o + patch] += 1
+        coverage *= int(cover.max())
+    if coverage * 2 ** (ACC_FRACTION_BITS + 1) >= 2 ** 63:
+        raise OverflowError("a voxel is covered by %d windows (patch %d, overlap %g): the fixed-point sums could overflow "
+                            "int64; use a smaller overlap" % (coverage, patch, overlap))
+    return axes
+
+
+def _first_conv_in(model):
+    return next(m.in_channels for m in model.modules() if isinstance(m, torch.nn.Conv3d))
+
+
+def _accumulate_windows(model, vol, patch, overlap, blend, sigma_scale, batch, graph, rank, world):
+    """Blended int64 accumulators [n_out * channels, D, H, W] of this rank's share of the windows (before any merge),
+    and the per-axis origin lists.  With ``graph`` the result is the static buffer of the captured pass: valid until the
+    next pass with the same configuration."""
+    d, h, w = vol.shape[1:]
+    axes = window_grid((d, h, w), patch, overlap)
+    origins = [(z, y, x) for z in axes[0] for y in axes[1] for x in axes[2]]
+    if world > 1:
+        from .parallel import shard_range
+        lo, hi = shard_range(len(origins), rank, world)
+        origins = origins[lo:hi]
+    sp = getattr(model, "_head_mode", "plain") != "plain"
+    nch = 4 if sp else model.last_conv.out_channels          # [out][channel]: SP heads have two outputs of two channels
+    org = torch.tensor(origins, dtype=torch.int32, device=vol.device).view(-1, 3)
+    nfull = (len(origins) // batch) * batch if graph else 0
+    if nfull:
+        st_vol, (acc, wt), st_org, g = _captured_fused_pass(model, vol, patch, batch, 2 if sp else 1,
+                                                            accum=(blend, sigma_scale, nch))
+        if st_vol.data_ptr() != vol.data_ptr():
+            st_vol.copy_(vol)
+    else:
+        st_vol, g = vol, None
+        acc = torch.empty((nch, d, h, w), dtype=torch.int64, device=vol.device)
+        wt = torch.tensor(window_weights(patch, blend, sigma_scale), dtype=torch.float32).expand(3, patch).contiguous()
+        wt = wt.to(vol.device)
+    acc.zero_()
+    for i in range(0, nfull, batch):
+        st_org.copy_(org[i:i + batch])
+        g.replay()
+    for i in range(nfull, len(origins), batch):          # a ragged last batch (or every batch without graph) runs eagerly
+        model.accumulate_windows(vol=st_vol, origins=org[i:i + batch], patch=patch, weights=wt, acc=acc)
+    return acc, axes
+
+
+@torch.no_grad()
+def sliding_window_predict(model, vol: torch.Tensor, patch: int = 128, overlap: float = 0.5, blend: str = "gaussian",
+                           sigma_scale: float = 0.125, batch: int = 4, graph: bool = True, probs: bool = False,
+                           rank: int = 0, world: int = 1, group=None):
+    """Eval-mode model over overlapping ``patch``^3 windows of ``vol`` float32 CUDA [Cin, D, H, W] of any size, the head
+    outputs blended with a constant or Gaussian importance map (semantics above).  Returns the float32 [D, H, W] label
+    volume(s), one per model output, as ``sliding_window_argmax`` does; with ``probs`` also returns the normalised blended
+    outputs, float32 [C, D, H, W] per output: ``(labels, probs)``.
+
+    Every full batch of windows replays one captured pass (gather -> network -> weighted sums into int64 accumulators),
+    a ragged tail runs eagerly, and one kernel finalizes.  ``world`` > 1: the windows are sharded over the ranks
+    (``parallel.shard_range``) and one all-reduce of the integer accumulators merges them, so every rank returns exactly
+    the single-rank result."""
+    if not isinstance(vol, torch.Tensor) or not vol.is_cuda:
+        raise RuntimeError("sliding_window_predict runs on CUDA tensors only (no CPU fallback)")
+    if vol.dtype != torch.float32:
+        raise TypeError("sliding_window_predict expects a float32 volume, got %s" % vol.dtype)
+    if vol.dim() != 4:
+        raise ValueError("expected [Cin, D, H, W]")
+    if not hasattr(model, "accumulate_windows"):
+        raise TypeError("sliding_window_predict needs a ctunet_b200 model (got %s)" % type(model).__name__)
+    if not 0.0 <= overlap < 1.0:
+        raise ValueError("overlap must be in [0, 1), got %r" % (overlap,))
+    if blend not in _BLENDS:
+        raise ValueError("blend must be one of %s, got %r" % (_BLENDS, blend))
+    if not sigma_scale > 0:
+        raise ValueError("sigma_scale must be > 0, got %r" % (sigma_scale,))
+    m = max(2 ** model._levels(), 4)
+    if patch <= 0 or patch % m:
+        raise ValueError("patch size %d must be a positive multiple of %d" % (patch, m))
+    if batch < 1:
+        raise ValueError("batch must be >= 1")
+    if vol.shape[0] != _first_conv_in(model):
+        raise ValueError("the volume has %d channels, the model takes %d" % (vol.shape[0], _first_conv_in(model)))
+    was_training = model.training
+    model.eval()
+    try:
+        vol = vol.contiguous()
+        acc, axes = _accumulate_windows(model, vol, patch, overlap, blend, sigma_scale, batch, graph, rank, world)
+        if world > 1:
+            import torch.distributed as dist
+            dist.all_reduce(acc, op=dist.ReduceOp.SUM, group=group)     # integer sums: the merge is exact
+        d, h, w = vol.shape[1:]
+        n_out = 2 if getattr(model, "_head_mode", "plain") != "plain" else 1
+        nch = acc.shape[0] // n_out
+        labels = [torch.empty((d, h, w), dtype=torch.float32, device=vol.device) for _ in range(n_out)]
+        blended, norm = [], None
+        if probs:
+            wt = window_weights(patch, blend, sigma_scale).astype(np.float32).astype(np.float64)   # the kernel's weights
+            norm = torch.from_numpy(np.concatenate([window_normaliser(s, patch, o, wt) for s, o in zip((d, h, w), axes)]))
+            norm = norm.to(vol.device)
+            blended = [torch.empty((nch, d, h, w), dtype=torch.float32, device=vol.device) for _ in range(n_out)]
+        call("ctu_window_finalize", acc.data_ptr(), n_out, nch, d, h, w, norm.data_ptr() if probs else None,
+             labels[0].data_ptr(), labels[1].data_ptr() if n_out == 2 else None,
+             blended[0].data_ptr() if probs else None, blended[1].data_ptr() if probs and n_out == 2 else None, stream_ptr())
+    finally:
+        model.train(was_training)
+    return (labels, blended) if probs else labels

@@ -64,7 +64,8 @@ int ctu_has_tensor_path(void);
 int ctu_pack_ncdhw(const float* src, void* dst, int dtype, int n, int c, long long spatial, ctu_stream stream);
 int ctu_unpack_ncdhw(const void* src, float* dst, int dtype, int n, int c, long long spatial, ctu_stream stream);
 /* sliding-window inference (BASELINE config 4): n patches of patch^3 voxels gathered from a float32 [c][vd][vh][vw] volume at
- * the DEVICE int[n][3] origins (z, y, x) into the blocked layout -- no host-side slicing / stacking */
+ * the DEVICE int[n][3] origins (z, y, x) into the blocked layout -- no host-side slicing / stacking.  patch % 4 == 0; any
+ * volume width and any origin: input voxels outside the volume read as 0 */
 int ctu_pack_patches(const float* vol, const int* origins, void* dst, int dtype, int n, int c, int vd, int vh, int vw, int patch,
                      ctu_stream stream);
 
@@ -231,6 +232,19 @@ int ctu_head_fwd(int dtype, const void* const* h_srcs, const int* h_src_channels
 int ctu_head_labels(int dtype, const void* const* h_srcs, const int* h_src_channels, int nsrc, const float* w, const float* bias,
                     int cout, int flags, const int* origins, int patch, int vd, int vh, int vw, float* labels0, float* labels1,
                     int n, long long spatial, ctu_stream stream);
+/* Overlapping sliding-window inference (DESIGN.md section 7b): the head of every patch^3 window at the DEVICE origins adds
+ * llrint(w * v * 2^40) to the int64 accumulators acc[out][c][vd][vh][vw] for each output channel value v (what
+ * ctu_head_fwd writes) of every window voxel inside the volume, with w = weights[z] * weights[patch + y] *
+ * weights[2*patch + x] (DEVICE float[3][patch]).  Integer atomics: the sums are independent of the order of the windows.
+ * The head must be bounded (softmax or sigmoid): every v lies in [0, 2]. */
+int ctu_head_accumulate(int dtype, const void* const* h_srcs, const int* h_src_channels, int nsrc, const float* w,
+                        const float* bias, int cout, int flags, const int* origins, int patch, int vd, int vh, int vw,
+                        const float* weights, long long* acc, int n, long long spatial, ctu_stream stream);
+/* labels[o] = float32 argmax over the channels of acc[o] (first maximum wins) for n_out = 1 or 2 outputs of `channels`
+ * channels each; probs[o] (nullable) = float32 [channels][vd][vh][vw] acc * 2^-40 / (nz[z] * ny[y] * nx[x]) with the
+ * DEVICE float64 normaliser tables norm = [nz (vd) | ny (vh) | nx (vw)]. */
+int ctu_window_finalize(const long long* acc, int n_out, int channels, int vd, int vh, int vw, const double* norm,
+                        float* labels0, float* labels1, float* probs0, float* probs1, ctu_stream stream);
 /* dsrcs[i] nullable; dw [cout][cin_total] and db [cout] are zeroed by the call.  dw = db = NULL: source gradients only;
  * every dsrcs[i] NULL: parameter gradients only (two launches that can run on different streams) */
 /* out0 / out1 (nullable): the outputs ctu_head_fwd produced; with them the plain-sigmoid SP head skips the logits */
