@@ -99,6 +99,9 @@ SIGNATURES = {
     "ctu_resample_nearest_u8": (I, [P, P, I, I, I, I, I, I, P]),
     "ctu_resample_nearest_index": (I, [P, I, I, P]),
     "ctu_resample_trilinear_f32": (I, [P, P, I, I, I, I, I, I, P]),
+    "ctu_components_workspace_bytes": (LL, [I, I, I, I]),
+    "ctu_label_components": (I, [I, P, I, I, I, I, I, P, P, P, LL, P]),
+    "ctu_filter_components": (I, [I, P, I, I, I, I, I, LL, P, P, LL, P]),
     "ctu_dice_coeff": (I, [P, P, I, I, LL, P, P, P]),
     "ctu_hausdorff_workspace_bytes": (LL, [I, I, I, I, I]),
     "ctu_hausdorff": (I, [P, P, I, I, I, I, I, D, P, LL, P, P]),

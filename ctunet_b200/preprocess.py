@@ -13,7 +13,7 @@ import math
 import numpy as np
 import torch
 
-from ._lib import call, stream_ptr
+from ._lib import call, load, stream_ptr
 from .utilities import hard_segm_from_tensor
 
 
@@ -41,6 +41,76 @@ def hu_threshold(hu: torch.Tensor, thr: int) -> torch.Tensor:
     out = torch.empty(hu.shape, dtype=torch.uint8, device=hu.device)
     call("ctu_hu_threshold", hu.data_ptr(), out.data_ptr(), hu.numel(), int(thr), stream_ptr())
     return out
+
+
+# ------------------------------------------------------------------------------------------------ connected components
+# Semantics (DESIGN.md section 7c; frozen by tests/components_oracle.py on top of scipy.ndimage.label): a voxel is
+# foreground when it is non-zero; connectivity 6 / 18 / 26 = generate_binary_structure(3, 1 / 2 / 3); components are
+# numbered 1..n per volume in the raster order of their first voxel (scipy's numbering).  Each volume of a [B, D, H, W]
+# input is labelled on its own.  No host synchronisation: counts stay on the device.
+_MASK_DTYPES = {torch.uint8: 1, torch.bool: 1, torch.float32: 4}      # CTU_MASK_U8 / CTU_MASK_F32
+_CONNECTIVITIES = (6, 18, 26)
+
+
+def _components_input(mask, connectivity, what):
+    """[B, D, H, W] contiguous view of ``mask`` and the C-ABI dtype code; every argument error raises before a launch."""
+    if connectivity not in _CONNECTIVITIES:
+        raise ValueError("%s: connectivity must be 6, 18 or 26, got %r" % (what, connectivity))
+    if not isinstance(mask, torch.Tensor):
+        raise RuntimeError("%s runs on CUDA tensors only (no CPU fallback)" % what)
+    if mask.dim() not in (3, 4):
+        raise ValueError("%s expects a [D, H, W] or [B, D, H, W] volume, got %d dimensions" % (what, mask.dim()))
+    if mask.dtype not in _MASK_DTYPES:
+        raise TypeError("%s expects uint8, bool or float32, got %s" % (what, mask.dtype))
+    if mask.numel() >= 2 ** 31:
+        raise ValueError("%s: %d voxels; B*D*H*W must be below 2^31" % (what, mask.numel()))
+    if not mask.is_cuda:
+        raise RuntimeError("%s runs on CUDA tensors only (no CPU fallback)" % what)
+    m = mask.contiguous()
+    return (m if m.dim() == 4 else m.unsqueeze(0)), _MASK_DTYPES[mask.dtype]
+
+
+def _components_workspace(m):
+    nbytes = load().ctu_components_workspace_bytes(*m.shape)
+    return torch.empty(nbytes, dtype=torch.uint8, device=m.device), nbytes
+
+
+def label_components(mask: torch.Tensor, connectivity: int = 6):
+    """``scipy.ndimage.label`` on the device: (labels int32 like ``mask``, counts int64 [B] -- 0-dim for a [D, H, W]
+    input -- the number of components per volume).  ``mask``: uint8, bool or float32 CUDA tensor."""
+    m, code = _components_input(mask, connectivity, "label_components")
+    labels = torch.empty(m.shape, dtype=torch.int32, device=m.device)
+    counts = torch.zeros(m.shape[0], dtype=torch.int64, device=m.device)
+    if m.numel():
+        ws, nbytes = _components_workspace(m)
+        call("ctu_label_components", code, m.data_ptr(), *m.shape, connectivity, labels.data_ptr(), counts.data_ptr(),
+             ws.data_ptr(), nbytes, stream_ptr())
+    if mask.dim() == 3:
+        return labels[0], counts[0]
+    return labels, counts
+
+
+def _filter_components(mask, connectivity, min_size, what):
+    m, code = _components_input(mask, connectivity, what)
+    out = torch.empty_like(m)
+    if m.numel():
+        ws, nbytes = _components_workspace(m)
+        call("ctu_filter_components", code, m.data_ptr(), *m.shape, connectivity, min_size, out.data_ptr(), ws.data_ptr(),
+             nbytes, stream_ptr())
+    return out.view(mask.shape)
+
+
+def largest_component(mask: torch.Tensor, connectivity: int = 6) -> torch.Tensor:
+    """``mask`` with every voxel outside the largest component of its volume set to 0 (ties: the component whose first
+    voxel comes first in raster order, i.e. the lower label).  Same dtype and shape; an empty volume stays empty."""
+    return _filter_components(mask, connectivity, -1, "largest_component")
+
+
+def remove_small_components(mask: torch.Tensor, min_size: int, connectivity: int = 6) -> torch.Tensor:
+    """``mask`` with the voxels of every component smaller than ``min_size`` voxels set to 0.  Same dtype and shape."""
+    if int(min_size) != min_size or min_size < 0:
+        raise ValueError("remove_small_components: min_size must be a non-negative integer, got %r" % (min_size,))
+    return _filter_components(mask, connectivity, int(min_size), "remove_small_components")
 
 
 def resample_nearest(vol: torch.Tensor, out_size) -> torch.Tensor:

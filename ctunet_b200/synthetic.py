@@ -23,6 +23,24 @@ def skull_phantom(size: int, seed: int, device) -> torch.Tensor:
     return ((r >= 1.0 - thick) & (r <= 1.0)).to(torch.uint8)
 
 
+def head_ct_hu(shape=(256, 512, 512), seed: int = 0, device="cuda") -> torch.Tensor:
+    """int16 HU head CT: the phantom of scripts/bench_infer.py (brain at 40 HU in an ellipsoidal 1000 HU bone shell,
+    Gaussian noise of 30 HU) plus what a bone threshold of a real scan also keeps: a scanner-table slab under the head
+    (600 HU, not touching it) and sparse metal speckle (1500 HU, about one voxel in 10^4).  Thresholded at 300 HU it
+    holds one large component (the skull), one slab and thousands of islands."""
+    d, h, w = shape
+    g = torch.Generator(device=device).manual_seed(seed)
+    zz, yy, xx = torch.meshgrid(*[torch.linspace(-1, 1, n, device=device) for n in (d, h, w)], indexing="ij")
+    r = torch.sqrt((zz / 0.8) ** 2 + (yy / 0.88) ** 2 + (xx / 0.72) ** 2)
+    hu = torch.full(shape, -1000.0, device=device)
+    hu[r <= 1.0] = 40
+    hu[(r >= 0.93) & (r <= 1.0)] = 1000
+    hu[(yy >= 0.95) & (yy <= 0.98) & (xx.abs() <= 0.9)] = 600
+    del zz, yy, xx, r
+    hu[torch.rand(shape, device=device, generator=g) < 1e-4] = 1500
+    return (hu + 30 * torch.randn(shape, device=device, generator=g)).clamp(-1024, 3071).to(torch.int16)
+
+
 def make_training_batch(batch: int, in_channels: int, size: int, seed: int, device="cuda"):
     """(image [B,Cin,S,S,S] float32 {0,1}, (skull_onehot, flap_onehot) each [B,2,S,S,S] float32)."""
     random.seed(seed)

@@ -329,6 +329,24 @@ int ctu_resample_nearest_index(int* idx, int out_size, int in_size, ctu_stream s
 int ctu_resample_trilinear_f32(const float* src, float* dst, int sd, int sh, int sw, int dd, int dh, int dw,
                                ctu_stream stream);
 
+/* ---- connected components of [b][d][h][w] volumes (scipy.ndimage.label semantics; DESIGN.md section 7c).  A voxel is
+ *      foreground when it is non-zero; in_dtype is CTU_MASK_U8 (uint8 or bool) or CTU_MASK_F32 (float32, e.g. the label
+ *      volumes of the sliding-window functions).  connectivity 6, 18 or 26 = generate_binary_structure(3, 1 / 2 / 3);
+ *      b*d*h*w < 2^31.  Each volume is labelled on its own.  ws: caller-owned DEVICE scratch of
+ *      ctu_components_workspace_bytes(b, d, h, w) bytes, 16-byte aligned (-1: invalid shape). */
+#define CTU_MASK_U8 1
+#define CTU_MASK_F32 4
+long long ctu_components_workspace_bytes(int b, int d, int h, int w);
+/* labels int32 [b][d][h][w]: 0 background, components 1..n per volume in the raster order of their first voxel;
+ * counts int64 [b] = n per volume. */
+int ctu_label_components(int in_dtype, const void* in, int b, int d, int h, int w, int connectivity, int* labels,
+                         long long* counts, void* ws, long long ws_bytes, ctu_stream stream);
+/* out (same dtype and shape as in) = in, except 0 on the voxels of dropped components.  min_size >= 0: keep every
+ * component of at least min_size voxels; min_size < 0: keep only the largest component of each volume (ties: the one
+ * whose first voxel comes first in raster order). */
+int ctu_filter_components(int in_dtype, const void* in, int b, int d, int h, int w, int connectivity, long long min_size,
+                          void* out, void* ws, long long ws_bytes, ctu_stream stream);
+
 /* ---- reporting metrics of the loss handlers (utilities.py:53-70; ProblemHandler.py:84-88, 277-295) on fp32 NCDHW
  *      prediction / one-hot target pairs [b][c][spatial], 2 <= c <= 4.  monai (undeclared, unpinned in the reference) is
  *      restated: PARITY UNPINNED, the CPU statement is oracle/ref_stubs/monai/metrics.py. -------------------------------- */
