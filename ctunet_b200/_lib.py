@@ -105,6 +105,8 @@ SIGNATURES = {
     "ctu_dice_coeff": (I, [P, P, I, I, LL, P, P, P]),
     "ctu_hausdorff_workspace_bytes": (LL, [I, I, I, I, I]),
     "ctu_hausdorff": (I, [P, P, I, I, I, I, I, D, P, LL, P, P]),
+    "ctu_surface_metrics_workspace_bytes": (LL, [I, I, I, I, I]),
+    "ctu_surface_metrics": (I, [I, P, I, P, I, I, I, I, P, D, D, P, P, LL, P]),
     "ctu_loss_combine": (I, [P, P, I, P, P, P]),
     "ctu_optim_chunk_bytes": (I, []),
     "ctu_optim_chunk_elems": (I, []),

@@ -6,6 +6,8 @@
   SkullRandomHole         ctunet/pytorch/transforms.py:52-94
   encode_flaprec_batch    ctunet/pytorch/datasets.py:195-235, :30-47 (one-hot targets, atlas channel)
   dice_coeff, hausdorff   ctunet/utilities.py:53-70 (reporting metrics; monai restated -> parity unpinned)
+  surface_metrics         no reference counterpart: per-volume Dice, Hausdorff, percentile Hausdorff, ASSD and surface
+                          Dice with voxel spacing (DESIGN.md section 7d; oracle tests/surface_oracle.py)
   SaltAndPepper           ctunet/pytorch/transforms.py:13-49
 
 The 'flap' shape of shape_3d calls the un-vendored, unpinned ``raster_geometry`` package in the reference
@@ -15,6 +17,8 @@ the flap shape is parity unpinned.
 """
 from __future__ import annotations
 
+import ctypes
+import math
 import random
 
 import numpy as np
@@ -269,6 +273,71 @@ def hausdorff(result_b: torch.Tensor, reference_b: torch.Tensor) -> torch.Tensor
     call("ctu_hausdorff", p.data_ptr(), t.data_ptr(), b, c, d, h, w, float(max(reference_b.shape)), ws.data_ptr(), nbytes,
          out.data_ptr(), stream_ptr())
     return out[0]
+
+
+_MASK_DTYPES = {torch.uint8: 1, torch.bool: 1, torch.float32: 4}      # CTU_MASK_U8 / CTU_MASK_F32
+SURFACE_METRIC_KEYS = ("dice", "hausdorff", "hausdorff_percentile", "assd", "surface_dice")
+
+
+def _number(x):
+    return isinstance(x, (int, float, np.integer, np.floating)) and not isinstance(x, bool)
+
+
+def surface_metrics(pred: torch.Tensor, target: torch.Tensor, spacing=None, percentile: float = 95.0,
+                    tolerance: float = 1.0) -> dict:
+    """Surface-distance scores of a binary prediction against its ground truth, per volume (DESIGN.md section 7d).
+
+    ``pred`` and ``target``: CUDA masks of one shape, [D, H, W] or [B, D, H, W], each uint8, bool or float32; a voxel is
+    foreground when it is non-zero (for several classes pass ``labels == k``); every axis at most 1024.  Edges are the
+    mask minus its 6-neighbourhood erosion (voxels outside the volume are background); d(A->B) are the Euclidean
+    distances from each edge voxel of A to the nearest edge voxel of B, in voxels, or in the unit of ``spacing`` =
+    (sz, sy, sx) in the D, H, W order.
+
+    Returns float64 CUDA tensors ([B], or 0-dim for a [D, H, W] input), computed without a host synchronisation:
+      dice                  2|P n T| / (|P| + |T|)
+      hausdorff             max(max d(P->T), max d(T->P))
+      hausdorff_percentile  max(pct(d(P->T)), pct(d(T->P))), pct = numpy.percentile(., percentile) (method "linear")
+      assd                  mean of d(P->T) and d(T->P) together
+      surface_dice          (#{d(P->T) <= tolerance} + #{d(T->P) <= tolerance}) / (#edges(P) + #edges(T))
+    Both masks empty: every value is NaN.  One mask empty: dice and surface_dice are 0, the three distances +inf (a
+    predicted structure that does not exist scores 0; unlike ``dice_coeff``, nothing is NaN)."""
+    what = "surface_metrics"
+    for t in (pred, target):
+        if not isinstance(t, torch.Tensor):
+            raise RuntimeError("%s runs on CUDA tensors only (no CPU fallback)" % what)
+    if pred.dim() not in (3, 4):
+        raise ValueError("%s expects [D, H, W] or [B, D, H, W] masks, got %d dimensions" % (what, pred.dim()))
+    if pred.shape != target.shape:
+        raise ValueError("%s: prediction %s and target %s differ in shape" % (what, tuple(pred.shape), tuple(target.shape)))
+    if not all(1 <= n <= 1024 for n in pred.shape[-3:]) or pred.numel() >= 2 ** 31:
+        raise ValueError("%s: every axis must be 1..1024 and B*D*H*W below 2^31, got %s" % (what, tuple(pred.shape)))
+    for t in (pred, target):
+        if t.dtype not in _MASK_DTYPES:
+            raise TypeError("%s expects uint8, bool or float32 masks, got %s" % (what, t.dtype))
+    sp = None
+    if spacing is not None:
+        sp = list(spacing) if isinstance(spacing, (tuple, list)) else None
+        if sp is None or len(sp) != 3 or not all(_number(s) and math.isfinite(s) and s > 0 for s in sp):
+            raise ValueError("%s: spacing must be three positive finite numbers (sz, sy, sx), got %r" % (what, spacing))
+        sp = [float(s) for s in sp]
+    if not _number(percentile) or not 0 <= percentile <= 100:
+        raise ValueError("%s: percentile must be in [0, 100], got %r" % (what, percentile))
+    if not _number(tolerance) or not tolerance >= 0:
+        raise ValueError("%s: tolerance must be >= 0, got %r" % (what, tolerance))
+    if not pred.is_cuda or not target.is_cuda:
+        raise RuntimeError("%s runs on CUDA tensors only (no CPU fallback)" % what)
+    if pred.device != target.device:
+        raise ValueError("%s: prediction on %s, target on %s" % (what, pred.device, target.device))
+    p, t = pred.contiguous(), target.contiguous()
+    b = p.shape[0] if p.dim() == 4 else 1
+    d, h, w = p.shape[-3:]
+    nbytes = _load().ctu_surface_metrics_workspace_bytes(b, d, h, w, int(sp is not None))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=p.device)
+    out = torch.empty((5, b), dtype=torch.float64, device=p.device)
+    call("ctu_surface_metrics", _MASK_DTYPES[p.dtype], p.data_ptr(), _MASK_DTYPES[t.dtype], t.data_ptr(), b, d, h, w,
+         (ctypes.c_double * 3)(*sp) if sp is not None else None, float(percentile), float(tolerance), out.data_ptr(),
+         ws.data_ptr(), nbytes, stream_ptr())
+    return {k: (out[i] if p.dim() == 4 else out[i, 0]) for i, k in enumerate(SURFACE_METRIC_KEYS)}
 
 
 # ---------------------------------------------------------------------------------------------- SaltAndPepper

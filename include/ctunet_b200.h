@@ -361,6 +361,22 @@ long long ctu_hausdorff_workspace_bytes(int b, int c, int d, int h, int w);
 int ctu_hausdorff(const float* pred, const float* target, int b, int c, int d, int h, int w, double inf_alt, void* workspace,
                   long long workspace_bytes, double* out, ctu_stream stream);
 
+/* ---- surface-distance evaluation of binary masks (DESIGN.md section 7d).  pred and target: [b][d][h][w], each
+ *      CTU_MASK_U8 (uint8 or bool) or CTU_MASK_F32, non-zero = foreground; every axis 1..1024, b*d*h*w < 2^31.  Edges are
+ *      the mask minus its 6-neighbourhood erosion (outside = background); d(A->B) = the Euclidean distances from the edge
+ *      voxels of A to the nearest edge voxel of B, in voxel units (spacing NULL) or weighted by spacing = host double[3]
+ *      (sz, sy, sx), positive and finite.  out: DEVICE double[5][b], rows dice (2|P n T| / (|P| + |T|)), hausdorff (max of
+ *      both directed maxima), hausdorff_percentile (max over both directions of numpy.percentile(d, percentile), method
+ *      "linear"), assd (mean of both directed distance sets together), surface_dice (#{d <= tolerance} over both
+ *      directions / (#edges(P) + #edges(T))).  Both masks empty: all NaN; one empty: dice and surface_dice 0, distances
+ *      +inf.  0 <= percentile <= 100, tolerance >= 0.  No host synchronisation; the same inputs give the same bits.
+ *      ws: DEVICE scratch of ctu_surface_metrics_workspace_bytes(b, d, h, w, spacing != NULL) bytes, 8-byte aligned
+ *      (-1: invalid shape). */
+long long ctu_surface_metrics_workspace_bytes(int b, int d, int h, int w, int weighted);
+int ctu_surface_metrics(int pred_dtype, const void* pred, int target_dtype, const void* target, int b, int d, int h, int w,
+                        const double* spacing, double percentile, double tolerance, double* out, void* ws, long long ws_bytes,
+                        ctu_stream stream);
+
 /* ---- the tail of a training iteration (Model.py:366-371, 510-546; ProblemHandler.py:59-91, 241-298) -------------------
  * comps[i] = lambdas[i] * *terms[i] (device scalars, host array of pointers), comps[n] = their sum in order; mirror
  * (nullable) receives a second copy (the tail of the data-parallel flat gradient buffer). */
