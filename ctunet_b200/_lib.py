@@ -122,6 +122,9 @@ SIGNATURES = {
     "ctu_optim_step_peer": (I, [I, P, I, P, P, I, I, P, P, P, P, P, D, D, D, D, D, D, I, D, P, LL, I, P]),
     "ctu_peer_error": (I, [P]),
     "ctu_salt_pepper_u8": (I, [P, P, LL, D, D, P, P, ULL, ULL, P]),
+    "ctu_affine_draw": (I, [I, I, I, I, P, I, ULL, P, P, P, P]),
+    "ctu_affine_encode_flaprec": (I, [I, P, P, P, P, P, P, P, P, I, I, I, I, I, P]),
+    "ctu_affine_masks_u8": (I, [I, P, P, P, I, I, I, I, P]),
 }
 
 _lib = None

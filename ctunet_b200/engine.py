@@ -139,6 +139,18 @@ def _splitmix64(x: int) -> int:
     return x ^ (x >> 31)
 
 
+def philox_key(device, domain: int = 0) -> int:
+    """64-bit Philox key of one random stream on ``device``: ``torch.initial_seed()`` mixed with the device index, the
+    ``torch.distributed`` rank (when one is initialised) and ``domain``, a constant per consumer (0: Dropout3d) so that
+    streams of different consumers never share a key."""
+    device = torch.device(device)
+    rank = 0
+    if torch.distributed.is_available() and torch.distributed.is_initialized():
+        rank = torch.distributed.get_rank()
+    idx = device.index if device.index is not None else torch.cuda.current_device()
+    return _splitmix64(torch.initial_seed() ^ _splitmix64(((idx << 32) | (rank & 0xFFFFFFFF)) ^ domain))
+
+
 class DropoutRNG:
     """Random state of the Dropout3d sites of one model on one device: a 64-bit Philox key and the pass counter, which
     lives in device memory and is advanced by the mask launch itself (ctu_dropout3d_keep), so a captured step draws new
@@ -148,12 +160,7 @@ class DropoutRNG:
     __slots__ = ("key", "counter", "last")
 
     def __init__(self, device):
-        device = torch.device(device)
-        rank = 0
-        if torch.distributed.is_available() and torch.distributed.is_initialized():
-            rank = torch.distributed.get_rank()
-        idx = device.index if device.index is not None else torch.cuda.current_device()
-        self.key = _splitmix64(torch.initial_seed() ^ _splitmix64((idx << 32) | (rank & 0xFFFFFFFF)))
+        self.key = philox_key(device)
         self.counter = torch.zeros(1, dtype=torch.int64, device=device)
         self.last = {}          # site name -> [N, C] view of the keep factors of the last pass that drew masks
 

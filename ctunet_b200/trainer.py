@@ -112,13 +112,23 @@ class TrainStep:
     ``optimizer``: 'adam' | 'adamw' (amsgrad=True) | 'rmsprop' | 'sgd' with the reference's arguments (Model.py:514-541);
     ``scheduler=True`` (or a dict of ReduceLROnPlateau arguments): ``ReduceLROnPlateau()`` stepped after every iteration on that iteration's total loss (Model.py:369-371,
     544-546).  Data parallel: pass ``grad_sync=GradSync(model, ...)``; the loss every rank logs and feeds the scheduler is
-    the mean over ranks (what the reference computes on the gathered batch)."""
+    the mean over ranks (what the reference computes on the gathered batch).
+
+    ``augment=utilities.RandomAffine(...)``: ``step_from_masks`` / ``step_from_bits`` draw one random affine transform per
+    sample and encode the transformed masks straight into the step's inputs (``ctu_affine_encode_flaprec``; the atlas
+    channel stays as it is), outside the captured graph like the plain encoders; ``last_affine()`` returns what the latest
+    step drew.  Such a step takes masks only: ``__call__`` with a ready image raises ``ValueError``."""
 
     def __init__(self, model, handler: str = "double", dice_lambda: float = 1.0, ce_lambda: float = 1.0,
                  lr: float = 1e-4, weight_decay: float = 0.0, optimizer: str = "adam", momentum: float = 0.99,
                  scheduler=False, grad_sync: Optional[GradSync] = None, input_requires_grad: bool = True,
-                 graph: bool = False, split_graph: Optional[bool] = None):
+                 graph: bool = False, split_graph: Optional[bool] = None, augment=None):
+        from .utilities import RandomAffine
+        if augment is not None and not isinstance(augment, RandomAffine):
+            raise TypeError("augment: a utilities.RandomAffine or None")
         self.model = model
+        self.augment = augment
+        self._last_affine = None                              # (params, matrices) of the latest augmenting step
         self.spec = _LossSpec(handler, dice_lambda, ce_lambda)
         self.handler, self.keys = handler, self.spec.keys
         self.input_requires_grad = input_requires_grad       # Model.py:351-352
@@ -191,6 +201,11 @@ class TrainStep:
         return comps
 
     def __call__(self, image: torch.Tensor, target):
+        if self.augment is not None:
+            raise ValueError("an augmenting TrainStep transforms masks: feed it through step_from_masks / step_from_bits")
+        return self._step(image, target)
+
+    def _step(self, image: torch.Tensor, target):
         if not self.graph:
             return self._eager(image, target)
         self._calls += 1
@@ -260,6 +275,10 @@ class TrainStep:
         if self.handler != "double":
             raise ValueError("step_from_masks feeds the double-output handler (full skull + flap targets)")
         masks = FUSED_HEAD_LOSS and (self._graph is None or self._static[1].dtype == torch.uint8)
+        if self.augment is not None:
+            if not masks:
+                raise ValueError("an augmenting step feeds uint8 label masks to the fused head + loss kernels")
+            return self._augmented(0, (broken, full, flap), tuple(broken.shape[1:]), atlas)
         if self._graph is not None:
             if masks:
                 encode_flaprec_batch(broken, full, flap, atlas, out=(self._static[0], None))
@@ -273,9 +292,9 @@ class TrainStep:
             image = torch.empty((broken.shape[0], 1 if atlas is None else 2) + tuple(broken.shape[1:]), dtype=torch.float32,
                                 device=broken.device)
             encode_flaprec_batch(broken, full, flap, atlas, out=(image, None))
-            return self(image, (full.contiguous(), flap.contiguous()))
+            return self._step(image, (full.contiguous(), flap.contiguous()))
         image, target = encode_flaprec_batch(broken, full, flap, atlas)
-        return self(image, target)
+        return self._step(image, target)
 
     def step_from_bits(self, broken_bits: torch.Tensor, full_bits: torch.Tensor, flap_bits: torch.Tensor, vol_shape, atlas=None):
         """``step_from_masks`` for BIT-PACKED masks ([B, D*H*W/8] uint8 each on the device, ``utilities.pack_mask_bits``):
@@ -284,6 +303,8 @@ class TrainStep:
         from .utilities import encode_flaprec_bits
         if self.handler != "double" or not FUSED_HEAD_LOSS:
             raise ValueError("step_from_bits feeds the double-output handler through the fused head + loss kernels")
+        if self.augment is not None:
+            return self._augmented(1, (broken_bits, full_bits, flap_bits), tuple(vol_shape), atlas)
         if self._graph is not None:
             if self._static[1].dtype != torch.uint8:
                 raise RuntimeError("the step was captured with float targets: capture it through step_from_bits / step_from_masks")
@@ -291,7 +312,51 @@ class TrainStep:
                                 out=(self._static[0], (self._static[1], self._static[2])))
             return self._replay()
         image, masks = encode_flaprec_bits(broken_bits, full_bits, flap_bits, vol_shape, atlas)
-        return self(image, masks)
+        return self._step(image, masks)
+
+    def _augmented(self, bits: int, srcs, vol, atlas):
+        """Draw the batch's transforms and encode the transformed masks into the step's inputs (the captured graph's static
+        inputs once it exists): float image (+ the atlas, untransformed) and the two uint8 label masks."""
+        broken = srcs[0]
+        for t in srcs:
+            if not isinstance(t, torch.Tensor) or not t.is_cuda:
+                raise RuntimeError("the masks must be CUDA tensors (no CPU fallback)")
+            if t.dtype not in ((torch.uint8,) if bits else (torch.uint8, torch.bool)) or t.shape != broken.shape:
+                raise TypeError("three %s masks of one shape expected" % ("uint8 bit-packed [B, D*H*W/8]" if bits else
+                                                                         "uint8 [B, D, H, W]"))
+        if len(vol) != 3:
+            raise ValueError("vol_shape: (D, H, W)")
+        b = broken.shape[0]
+        d, h, w = (int(v) for v in vol)
+        if (broken.dim() != 2 or broken.shape[1] * 8 != d * h * w) if bits else (broken.dim() != 4 or tuple(broken.shape[1:]) != vol):
+            raise ValueError("masks %s do not match the volume shape %s" % (tuple(broken.shape), vol))
+        cin = 1 if atlas is None else 2
+        if atlas is not None and (atlas.dtype != torch.float32 or tuple(atlas.shape) != (d, h, w) or not atlas.is_cuda):
+            raise TypeError("atlas: float32 CUDA volume of the mask shape")
+        if self._graph is not None:
+            if self._static[1].dtype != torch.uint8:
+                raise ValueError("the step was captured with float targets: an augmenting step needs uint8 label masks")
+            image, fm, lm = self._static
+            if tuple(image.shape) != (b, cin, d, h, w):
+                raise RuntimeError("graph mode: the batch shape changed after the step was captured")
+        else:
+            image = torch.empty((b, cin, d, h, w), dtype=torch.float32, device=broken.device)
+            fm = torch.empty((b, d, h, w), dtype=torch.uint8, device=broken.device)
+            lm = torch.empty_like(fm)
+        params, mats = self.augment.draw(b, (d, h, w), broken.device)
+        src = [t.contiguous() for t in srcs]
+        call("ctu_affine_encode_flaprec", bits, *[t.data_ptr() for t in src],
+             atlas.contiguous().data_ptr() if atlas is not None else None, mats.data_ptr(), image.data_ptr(), fm.data_ptr(),
+             lm.data_ptr(), b, cin, d, h, w, stream_ptr())
+        self._last_affine = (params, mats)
+        if self._graph is not None:
+            return self._replay()
+        return self._step(image, (fm, lm))
+
+    def last_affine(self):
+        """``(params [B, 10], matrices [B, 3, 4])`` the latest augmenting step drew (``RandomAffine.draw``), or None; valid
+        until the next step."""
+        return self._last_affine
 
     @property
     def lr(self) -> float:

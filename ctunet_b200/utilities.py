@@ -9,6 +9,8 @@
   surface_metrics         no reference counterpart: per-volume Dice, Hausdorff, percentile Hausdorff, ASSD and surface
                           Dice with voxel spacing (DESIGN.md section 7d; oracle tests/surface_oracle.py)
   SaltAndPepper           ctunet/pytorch/transforms.py:13-49
+  RandomAffine,           no reference counterpart: seeded rotation, scaling, translation and flips of mask batches
+  affine_masks            (DESIGN.md section 7e; oracle tests/affine_oracle.py)
 
 The 'flap' shape of shape_3d calls the un-vendored, unpinned ``raster_geometry`` package in the reference
 (utilities.py:145-166); it is not installed here, so ``cylinder`` / ``cube`` are RESTATED from the package's published
@@ -24,7 +26,7 @@ import random
 import numpy as np
 import torch
 
-from ._lib import call, stream_ptr
+from ._lib import call, ptr_array, stream_ptr
 from ._lib import load as _load
 from .losses import dice_loss  # noqa: F401  (re-export: utils.dice_loss)
 
@@ -387,3 +389,141 @@ class SaltAndPepper(object):
             out = out.float()
             sample[keyw] = out if is_batch else out[0]
         return sample
+
+
+# ---------------------------------------------------------------------------------------------- RandomAffine
+AFFINE_DOMAIN = 0xAFF1            # engine.philox_key domain of the affine draws (Dropout3d uses 0)
+AFFINE_PARAM_KEYS = ("angle_d", "angle_h", "angle_w", "scale", "shift_z", "shift_y", "shift_x", "flip_z", "flip_y", "flip_x")
+
+
+def _triple(v, what):
+    t = tuple(v) if isinstance(v, (tuple, list)) else (v, v, v)
+    if len(t) != 3 or not all(_number(x) and math.isfinite(x) for x in t):
+        raise ValueError("%s must be a finite number or a (d, h, w) triple, got %r" % (what, v))
+    return tuple(float(x) for x in t)
+
+
+def _mask_batch(masks, what):
+    """Validate a list of 1..3 uint8 / bool CUDA masks of one [B, D, H, W] shape (errors before any launch)."""
+    if not isinstance(masks, (tuple, list)) or not 1 <= len(masks) <= 3:
+        raise ValueError("%s expects a list of 1 to 3 masks" % what)
+    for m in masks:
+        if not isinstance(m, torch.Tensor):
+            raise TypeError("%s expects tensors, got %s" % (what, type(m).__name__))
+        if m.dim() != 4 or m.shape != masks[0].shape:
+            raise ValueError("%s expects masks of one [B, D, H, W] shape, got %s" % (what, [tuple(t.shape) for t in masks]))
+        if m.dtype not in (torch.uint8, torch.bool):
+            raise TypeError("%s expects uint8 or bool masks, got %s" % (what, m.dtype))
+    for m in masks:
+        if not m.is_cuda or m.device != masks[0].device:
+            raise RuntimeError("%s runs on CUDA tensors of one device only (no CPU fallback)" % what)
+
+
+def _check_matrices(matrices, batch, device, what):
+    if not isinstance(matrices, torch.Tensor) or matrices.dtype != torch.float32 or tuple(matrices.shape) != (batch, 3, 4):
+        raise ValueError("%s: matrices must be a float32 [%d, 3, 4] tensor, got %s" % (
+            what, batch, (matrices.dtype, tuple(matrices.shape)) if isinstance(matrices, torch.Tensor) else type(matrices)))
+    if not matrices.is_cuda or matrices.device != device:
+        raise RuntimeError("%s: the matrices must be on the masks' device %s" % (what, device))
+
+
+def affine_masks(masks, matrices):
+    """Transform 1 to 3 uint8 or bool CUDA masks [B, D, H, W] of one shape with the per-sample affine maps ``matrices``
+    (float32 [B, 3, 4], e.g. ``RandomAffine.draw``): nearest neighbour, a source outside the volume reads 0, every mask of
+    a sample takes the same source voxel (DESIGN.md section 7e).  Returns new masks of the input dtype and shape.  The
+    matrix values are not checked (that would synchronise): a non-finite source coordinate reads 0."""
+    _mask_batch(masks, "affine_masks")
+    b, d, h, w = masks[0].shape
+    _check_matrices(matrices, b, masks[0].device, "affine_masks")
+    src = [m.contiguous() for m in masks]
+    out = [torch.empty_like(m) for m in src]
+    u8 = lambda t: t.view(torch.uint8)          # noqa: E731  (bool is one byte of 0 / 1)
+    call("ctu_affine_masks_u8", len(src), ptr_array([u8(t).data_ptr() for t in src]),
+         ptr_array([u8(t).data_ptr() for t in out]), matrices.contiguous().data_ptr(), b, d, h, w, stream_ptr())
+    return out
+
+
+class RandomAffine(object):
+    """Random rotation, isotropic scaling, translation and flips of training masks on the device (DESIGN.md section 7e).
+
+    ``rotate``: degrees, a number or a (d, h, w) triple; the angle about each axis is uniform in [-r, r], 0 <= r <= 180.
+    ``scale``: (lo, hi), the scale is uniform in [lo, hi].  ``translate``: voxels, a number or a (z, y, x) triple; uniform
+    in [-T, T].  ``flip``: per axis (d, h, w), an enabled axis flips with probability 1/2 (default: left-right only, the one
+    symmetry of a skull).  ``RandomAffine(0, (1, 1), 0, (False, False, False))`` is the identity.
+
+    Each sample's map sends output voxel p to source q = c + t + (1/s) R F (p - c) about the volume centre c, sampled with
+    nearest neighbour, so binary masks stay binary and ``broken & flap == 0``, ``broken | flap == full`` are kept exactly.
+    The draws come from a Philox stream on the device (``ctu_affine_draw``): the key is ``torch.initial_seed()`` when the
+    transform first draws on a device, mixed with the device index, the ``torch.distributed`` rank and a constant of its
+    own (``engine.philox_key``); the pass counter lives in device memory and each draw advances it.
+    ``torch.manual_seed(s)`` before the first draw reproduces a run, ranks draw independent transforms.
+
+    ``__call__(sample)`` takes the dict of ``SkullRandomHole`` (uint8 / bool CUDA ``image`` [B, D, H, W] or [D, H, W], a
+    mask or a tuple of masks as ``target``), so ``RandomAffine()(SkullRandomHole(double_output=True)(s))`` composes.  The
+    atlas channel of a shape-prior model is NOT transformed: it is the fixed prior in atlas space, and the misregistration
+    between it and the skull is what the augmentation simulates (``TrainStep(augment=...)`` leaves it as it is)."""
+
+    def __init__(self, rotate=15.0, scale=(0.9, 1.1), translate=8.0, flip=(False, False, True)):
+        rot = _triple(rotate, "rotate")
+        if not all(0 <= r <= 180 for r in rot):
+            raise ValueError("rotate must be in [0, 180] degrees, got %r" % (rotate,))
+        if not isinstance(scale, (tuple, list)) or len(scale) != 2 or not all(_number(x) and math.isfinite(x) for x in scale) \
+                or not 0 < scale[0] <= scale[1] <= 1000:
+            raise ValueError("scale must be (lo, hi) with 0 < lo <= hi <= 1000, got %r" % (scale,))
+        tr = _triple(translate, "translate")
+        if not all(0 <= t <= 1e6 for t in tr):
+            raise ValueError("translate must be in [0, 1e6] voxels, got %r" % (translate,))
+        if not isinstance(flip, (tuple, list)) or len(flip) != 3 or not all(isinstance(f, (bool, np.bool_)) for f in flip):
+            raise ValueError("flip must be three booleans (d, h, w), got %r" % (flip,))
+        self.rotate, self.scale, self.translate, self.flip = rot, (float(scale[0]), float(scale[1])), tr, tuple(map(bool, flip))
+        # float32 ranges the kernel reads: angles in radians, rounded once
+        self._ranges = [float(np.float32(math.radians(r))) for r in rot] + [float(np.float32(x)) for x in self.scale] + \
+                       [float(np.float32(t)) for t in tr]
+        self._flip_axes = sum(1 << k for k, f in enumerate(self.flip) if f)
+        self._state = {}                   # device -> (key, int64 pass counter on the device)
+        self.last = None                   # (params [B, 10], matrices [B, 3, 4]) of the latest draw
+
+    def draw(self, batch: int, vol_shape, device):
+        """Draw one transform per sample: ``(params, matrices)`` float32 CUDA tensors [B, 10] (angles about d, h, w in
+        radians, scale, shifts along z, y, x in voxels, flip signs) and [B, 3, 4].  No host synchronisation."""
+        d, h, w = (int(v) for v in vol_shape)
+        device = torch.device(device)
+        if device.type != "cuda":
+            raise RuntimeError("RandomAffine draws on CUDA devices only (no CPU fallback)")
+        if device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        st = self._state.get(device)
+        if st is None:
+            from .engine import philox_key
+            st = self._state[device] = (philox_key(device, AFFINE_DOMAIN), torch.zeros(1, dtype=torch.int64, device=device))
+        params = torch.empty((batch, 10), dtype=torch.float32, device=device)
+        mats = torch.empty((batch, 3, 4), dtype=torch.float32, device=device)
+        with torch.cuda.device(device):
+            call("ctu_affine_draw", int(batch), d, h, w, (ctypes.c_float * 8)(*self._ranges), self._flip_axes, st[0],
+                 st[1].data_ptr(), params.data_ptr(), mats.data_ptr(), stream_ptr())
+        self.last = (params, mats)
+        return self.last
+
+    def __call__(self, sample):
+        img = sample["image"]
+        if not isinstance(img, torch.Tensor) or img.dtype not in (torch.uint8, torch.bool):
+            raise ValueError("RandomAffine transforms binary masks (uint8 / bool): encode float images after it")
+        tgt = sample.get("target")
+        tgts = list(tgt) if isinstance(tgt, (tuple, list)) else ([] if tgt is None else [tgt])
+        vols = [img] + tgts
+        is_batch = img.dim() == 4
+        if any(not isinstance(t, torch.Tensor) or t.dim() != img.dim() for t in vols) or img.dim() not in (3, 4):
+            raise ValueError("RandomAffine expects [D, H, W] or [B, D, H, W] masks of one shape")
+        batch = [t if is_batch else t.unsqueeze(0) for t in vols]
+        _mask_batch(batch, "RandomAffine")
+        _, mats = self.draw(batch[0].shape[0], batch[0].shape[1:], batch[0].device)
+        out = affine_masks(batch, mats)
+        if not is_batch:
+            out = [t[0] for t in out]
+        res = dict(sample)
+        res["image"] = out[0]
+        if isinstance(tgt, (tuple, list)):
+            res["target"] = type(tgt)(out[1:])
+        elif tgt is not None:
+            res["target"] = out[1]
+        return res

@@ -427,6 +427,30 @@ int ctu_salt_pepper_u8(const unsigned char* img, unsigned char* out, long long n
                        const double* u_black, const double* u_white, unsigned long long seed, unsigned long long offset,
                        ctu_stream stream);
 
+/* ---- random affine augmentation of mask batches (no reference counterpart: the reference has no spatial augmentation;
+ *      DESIGN.md section 7e).  Volumes [batch][d][h][w], 1 <= batch <= 65535, every axis below 2^22.
+ *      A sample's map from output voxel p = (z, y, x) to source point is q = c + t + (1/s) R F (p - c), c = (S - 1) / 2,
+ *      R = R_d(a_d) R_h(a_h) R_w(a_w) (R_a: rotation about axis a), F = diag(f_z, f_y, f_x), f = +-1; matrices = DEVICE
+ *      float[batch][3][4] rows (M_k0, M_k1, M_k2, M_k3).  Nearest neighbour in float32 without contraction:
+ *      q_k = ((M_k0 z + M_k1 y) + M_k2 x) + M_k3, i_k = floor(q_k + 0.5); the voxel reads 0 unless -0.5 < q_k < S_k - 0.5
+ *      on every axis (NaN / inf fail the test).  Every mask of a sample uses the same source index. ------------------ */
+/* params = DEVICE float[batch][10] (a_d, a_h, a_w in radians, s, t_z, t_y, t_x, f_z, f_y, f_x) and the matrices they give
+ * (built in double, rounded once).  h_ranges = HOST float[8]: max |angle| about d, h, w in [0, pi] (radians), scale lo,
+ * hi (0 < lo <= hi), max |translation| along z, y, x (voxels); angle = r (2u - 1), s = lo + (hi - lo) u, t = T (2u - 1),
+ * axis k flips when bit k of flip_axes is set and u < 0.5, u = 24-bit uniforms of Philox4x32-10 with counter = (pass,
+ * sample, call 0..2) and key = seed.  pass_counter: DEVICE int64 read, then advanced by the launch (NULL: pass 0). */
+int ctu_affine_draw(int batch, int d, int h, int w, const float* h_ranges, int flip_axes, unsigned long long seed,
+                    unsigned long long* pass_counter, float* params, float* matrices, ctu_stream stream);
+/* ctu_encode_flaprec_u8 (bits = 0: uint8 masks [batch][spatial]) / ctu_encode_flaprec_bits (bits = 1: bit-packed
+ * [batch * spatial / 8]) with the masks transformed: image channel 0 = transformed broken mask as float, channel 1 = the
+ * atlas UNCHANGED (the fixed shape prior in atlas space), full_mask / flap_mask = the transformed uint8 label masks. */
+int ctu_affine_encode_flaprec(int bits, const unsigned char* broken, const unsigned char* full, const unsigned char* flap,
+                              const float* atlas, const float* matrices, float* image, unsigned char* full_mask,
+                              unsigned char* flap_mask, int batch, int in_channels, int d, int h, int w, ctu_stream stream);
+/* the same gather for n = 1..3 uint8 masks: h_dst[i] = transformed h_src[i] (HOST arrays of device pointers) */
+int ctu_affine_masks_u8(int n, const unsigned char* const* h_src, unsigned char* const* h_dst, const float* matrices,
+                        int batch, int d, int h, int w, ctu_stream stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
