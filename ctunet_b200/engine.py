@@ -593,15 +593,7 @@ class Engine:
         if dw_out is not None:
             def wgrad_kernel():
                 dwp = self.wacc(lib.ctu_conv_wpack_floats(cout, k, ns, ca))
-                tc = 0
-                small = (self.use_tc and ns == 1 and not phase_cout
-                         and lib.ctu_conv_wide_wgrad_supported(k, srcs[0].c, cout, s0.d, s0.h, s0.w))
-                if small and max(s0.h, s0.w) <= WIDE_MAX_HW:
-                    tc = 2      # small grids: the tap-stationary kernel (8 x 8 plane tiles, d-planes split over CTAs)
-                elif self.use_tc and lib.ctu_conv_tc_wgrad_supported(k, ns, ca, cout, s0.d, s0.h, s0.w):
-                    tc = 1
-                elif small:
-                    tc = 2
+                tc = wgrad_variant(k, [s.c for s in srcs], cout, s0.d, s0.h, s0.w, phase_cout) if self.use_tc else 0
                 call("ctu_conv3d_wgrad", self.dtype, pa, ca, ns, dy.ptr, dwp.data_ptr(),
                      db_out.data_ptr() if db_out is not None else None, phase_cout, cout, k, s0.n, s0.d, s0.h, s0.w,
                      int(tc) | self._pz(dwp), stream_ptr())
@@ -1182,6 +1174,19 @@ def tc_variant(k, src_channels, cout, n, d, h, w) -> int:
         if not narrow or (min(chans[0], cout) >= WIDE_MIN_CH and max(h, w) <= WIDE_MAX_HW):
             return 2
     return 1 if narrow else 0
+
+
+def wgrad_variant(k, src_channels, cout, d, h, w, phase_cout=0) -> int:
+    """Which kernel computes the weight gradient of conv(cat(srcs)) -> cout on the tensor path: 0 none (CUDA cores),
+    1 conv_tc.cu (16-wide rows), 2 the tap-stationary small-grid kernel (8 x 8 plane tiles, d-planes split over CTAs)."""
+    lib = _lib.load()
+    chans = list(src_channels)
+    small = len(chans) == 1 and not phase_cout and lib.ctu_conv_wide_wgrad_supported(k, chans[0], cout, d, h, w)
+    if small and max(h, w) <= WIDE_MAX_HW:
+        return 2
+    if lib.ctu_conv_tc_wgrad_supported(k, len(chans), int_array(chans), cout, d, h, w):
+        return 1
+    return 2 if small else 0
 
 
 def tc_supported(k, src_channels, cout, d, h, w) -> bool:

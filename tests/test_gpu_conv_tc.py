@@ -58,6 +58,46 @@ def _bf(t):
     return t.to(torch.bfloat16).to(torch.float32)
 
 
+def _conv64(x, w, b, k):
+    """float64 conv3d(x, w) + b and its magnitude |w| (*) |x| + |b|, in d-slabs of at most 16 planes (plus the halo) so
+    that the float64 column buffers of the 128^3 cases stay small."""
+    p = k // 2
+    n, c, d, h, wd = x.shape
+    x, w = x.double(), w.double()
+    b = b.double() if b is not None else None
+    slab = max(1, min(16, (1 << 26) // (c * k ** 3 * h * wd)))
+    ys, bs = [], []
+    for z0 in range(0, d, slab):
+        z1 = min(d, z0 + slab)
+        lo, hi = max(0, z0 - p), min(d, z1 + p)
+        xs = F.pad(x[:, :, lo:hi], (0, 0, 0, 0, lo - (z0 - p), (z1 + p) - hi))
+        ys.append(F.conv3d(xs, w, b, 1, (0, p, p)))
+        bs.append(F.conv3d(xs.abs(), w.abs(), b.abs() if b is not None else None, 1, (0, p, p)))
+    return torch.cat(ys, 2), torch.cat(bs, 2)
+
+
+def _check_elementwise(got, x, w, b, k, what):
+    """|y - y64| <= 2^-8 |y64| + 2^-16 (|w| (*) |x| + |b|) per element, y64 the float64 result on the bf16-rounded operands:
+    one bf16 rounding of the output (at most 2^-8 relative) plus fp32 accumulation error.  Returns the worst ratio to the
+    bound (printed, so that the rounding model can be compared with what the B200 does)."""
+    ref, mag = _conv64(x, w, b, k)
+    err = (got.double() - ref).abs()
+    bound = 2.0 ** -8 * ref.abs() + 2.0 ** -16 * mag
+    ratio = torch.where(bound > 0, err / bound.clamp_min(1e-300), err * float("inf")).nan_to_num(0.0)
+    worst = ratio.max().item()
+    print("%s: worst |err| / bound %.3f" % (what, worst))
+    if worst > 1.0:
+        idx = tuple(int(i) for i in (ratio == ratio.max()).nonzero()[0])
+        raise AssertionError("%s: |err| %.3e > bound %.3e at %s (ratio %.3f)" % (what, err[idx].item(), bound[idx].item(),
+                                                                                 idx, worst))
+    return worst
+
+
+def _dgrad_weights(w):
+    """The data gradient is a convolution of dy with the flipped, transposed weights."""
+    return w.flip(2, 3, 4).transpose(0, 1)
+
+
 @pytest.mark.parametrize("case", CASES + WIDE_CASES)
 def test_tc_conv_matches_reference(case):
     from ctunet_b200.engine import Engine, tc_variant
@@ -75,9 +115,6 @@ def test_tc_conv_matches_reference(case):
     wt = torch.randn(cout, cin, k, k, k, generator=g) / (cin * k ** 3) ** 0.5
     bs = torch.randn(cout, generator=g) if use_bias else None
     dy = _bf(torch.randn(n, cout, d, h, w, generator=g))
-    xr = x.clone().requires_grad_()
-    yr = F.conv3d(xr, _bf(wt) if fprop_on_tc else wt, bs, 1, k // 2)   # the tensor path rounds the weights to bf16
-    yr.backward(dy)
 
     eng = Engine(torch.device(DEV), "bf16", record=True)
     assert eng.use_tc
@@ -86,9 +123,8 @@ def test_tc_conv_matches_reference(case):
     xa = eng.pack(x.to(DEV))
     y = eng.conv([xa], wg, bg, k, [True], bn_stats=True)
     yo = eng.unpack(y).cpu()
-    scale = yr.abs().max().item()
-    err = (yo - yr.detach()).abs().max().item()
-    assert err <= 1e-2 * scale, "fprop err %.3e (scale %.3e)" % (err, scale)
+    scale = yo.abs().max().item()
+    _check_elementwise(yo, x, _bf(wt), bs, k, "fprop %s" % (case,))     # the tensor path rounds the weights to bf16
     # fused BatchNorm statistics = sums of the stored (bf16-rounded) outputs
     sums = y.sums.cpu()
     cpad = (cout + 7) // 8 * 8
@@ -100,9 +136,7 @@ def test_tc_conv_matches_reference(case):
     eng.agrads[id(y)] = eng.pack(dy.to(DEV))
     eng.run_tape()
     dx = eng.unpack(eng.agrads[id(xa)]).cpu()
-    gs = xr.grad.abs().max().item()
-    gerr = (dx - xr.grad).abs().max().item()
-    assert gerr <= 1.2e-2 * gs, "dgrad err %.3e (scale %.3e)" % (gerr, gs)
+    _check_elementwise(dx, dy, _dgrad_weights(_bf(wt)), None, k, "dgrad %s" % (case,))
     # weight gradient on the tensor cores (voxels as the K dimension): bf16 products, fp32 accumulation
     assert _lib.load().ctu_conv_tc_wgrad_supported(k, 1, _lib.int_array([cin]), cout, d, h, w) == (1 if h % 16 == 0 else 0)
     assert h % 16 == 0 or _lib.load().ctu_conv_wide_wgrad_supported(k, cin, cout, d, h, w) == 1   # 8 x 8: tap-stationary kernel
@@ -195,14 +229,17 @@ def test_tc_conv_concatenated_sources(chans, cout):
     assert eng._tc_ok(k, acts, cout)
     y = eng.conv(acts, wg, None, k, [True] * len(acts), bn_stats=True)
     yo = eng.unpack(y).cpu()
-    assert (yo - yr.detach()).abs().max().item() <= 1e-2 * yr.abs().max().item()
+    _check_elementwise(yo, torch.cat(xs, 1), _bf(wt), None, k, "fprop %s -> %d" % (chans, cout))
     cpad = (cout + 7) // 8 * 8
     assert torch.allclose(y.sums.cpu()[:cout], yo.double().sum((0, 2, 3, 4)), rtol=1e-4, atol=1e-2 * yr.abs().max().item())
     assert torch.allclose(y.sums.cpu()[cpad:cpad + cout], (yo.double() ** 2).sum((0, 2, 3, 4)), rtol=1e-4, atol=1e-3)
     eng.agrads[id(y)] = eng.pack(dy.to(DEV))
     eng.run_tape()
-    for a, r in zip(acts, xr):
+    wd = _dgrad_weights(_bf(wt))
+    c0 = 0
+    for i, a in enumerate(acts):
         dx = eng.unpack(eng.agrads[id(a)]).cpu()
-        assert (dx - r.grad).abs().max().item() <= 1.2e-2 * r.grad.abs().max().item()
+        _check_elementwise(dx, dy, wd[c0:c0 + chans[i]], None, k, "dgrad %s -> %d, source %d" % (chans, cout, i))
+        c0 += chans[i]
     dw = eng.pgrads[id(wg)].cpu()
     assert (dw - wr.grad).abs().max().item() <= 2e-3 * wr.grad.abs().max().item()
