@@ -12,7 +12,8 @@ from .losses import (dice_loss, dice_ce, ProblemHandler, FlapRec, FlapRecWithSha
                      FlapRecWithShapePriorDoubleOut, FlapRecDoubleOut)
 from .utilities import (hard_segm_from_tensor, shape_3d, blank_patch, random_blank_patch, encode_flaprec_batch,  # noqa: F401
                         SkullRandomHole, SaltAndPepper, kth_nonzero, count_nonzero, dice_coeff, hausdorff,
-                        surface_metrics, pack_mask_bits, encode_flaprec_bits, RandomAffine, affine_masks)
+                        surface_metrics, pack_mask_bits, encode_flaprec_bits, RandomAffine, affine_masks,
+                        RandomCraniectomy)
 from . import preprocess  # noqa: F401
 from .dropin import install, uninstall, MODEL_CLASSES, HANDLER_CLASSES  # noqa: F401
 

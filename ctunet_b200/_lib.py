@@ -125,6 +125,10 @@ SIGNATURES = {
     "ctu_affine_draw": (I, [I, I, I, I, P, I, ULL, P, P, P, P]),
     "ctu_affine_encode_flaprec": (I, [I, P, P, P, P, P, P, P, P, I, I, I, I, I, P]),
     "ctu_affine_masks_u8": (I, [I, P, P, P, I, I, I, I, P]),
+    "ctu_craniectomy_workspace_bytes": (LL, [I, I, I, I]),
+    "ctu_craniectomy_draw": (I, [I, P, I, I, I, I, D, I, I, I, ULL, P, P, P, LL, P]),
+    "ctu_craniectomy_encode_flaprec": (I, [I, P, P, P, P, P, P, P, I, I, I, I, I, P]),
+    "ctu_craniectomy_masks_u8": (I, [P, P, P, P, P, I, I, I, I, P]),
 }
 
 _lib = None

@@ -158,6 +158,48 @@ __device__ __forceinline__ double warp_sum(double v) {
     return v;
 }
 
+// ---------------------------------------------------------------- virtual-craniectomy inside tests
+// (transforms.py:286-296, utilities.py:127-178), shared by ctu_flap_mask_u8 (misc.cu) and the craniectomy encoder
+// (augment.cu).  Sphere (shape 0) / box (shape 1) with an INTEGER radius r (np.random.randint, transforms.py:268):
+// squared integer offsets are exact in I and sqrt is monotone, so np.linalg.norm(ord=2) <= r <=> dz^2 + dy^2 + dx^2 <= r^2
+// bit for bit; r < 0 leaves nothing inside.  I = int while every squared distance fits 31 bits.
+template <typename I>
+__device__ __forceinline__ bool ball_inside(int shape, I dz, I dy, I dx, I r) {
+    if (shape == 0) return r >= 0 && dz * dz + dy * dy + dx * dx <= r * r;
+    return (dz < 0 ? -dz : dz) <= r && (dy < 0 ? -dy : dy) <= r && (dx < 0 ? -dx : dx) <= r;
+}
+
+// shape_3d(shape="flap") (utilities.py:145-166): the union of two cylinders along d (raster_geometry.cylinder, axis 0)
+// and a cube (raster_geometry.cube).  raster_geometry is an un-vendored, unpinned dependency of the reference, so its
+// published algorithm is RESTATED -- parity unpinned: relative positions become absolute grid origins
+// x0 = rint((dim - 1) * rel) (round half to even), a cylinder is {(y-y0)^2 + (x-x0)^2 <= radius^2 and |z-z0| <= height/2},
+// a cube is {|c - c0| <= side/2 on every axis}, all in float64 (the offsets are integers, so the sums are exact).
+struct FlapHole {
+    double z0, ey, ex1, ex2, qy, qx, half, r2;
+};
+
+__device__ __forceinline__ FlapHole flap_hole(int d, int h, int w, double c0, double c1, double c2, double size,
+                                              double c_diam) {
+    FlapHole f;
+    // center_relative, z_edge_1, z_edge_2 (utilities.py:148-158) -> absolute origins
+    f.z0 = rint((d - 1) * (c0 / d));
+    f.ey = rint((h - 1) * ((c1 - size / 2) / h));
+    f.ex1 = rint((w - 1) * ((c2 - size / 2) / w));
+    f.ex2 = rint((w - 1) * ((c2 + size / 2) / w));
+    f.qy = rint((h - 1) * (c1 / h));
+    f.qx = rint((w - 1) * (c2 / w));
+    f.half = size / 2;
+    f.r2 = c_diam * c_diam;
+    return f;
+}
+
+__device__ __forceinline__ bool flap_inside(const FlapHole& f, double z, double y, double x) {
+    const bool in_height = fabs(z - f.z0) <= f.half;
+    const double dy = y - f.ey, dy2 = dy * dy;
+    return in_height && ((dy2 + (x - f.ex1) * (x - f.ex1) <= f.r2) || (dy2 + (x - f.ex2) * (x - f.ex2) <= f.r2) ||
+                         (fabs(y - f.qy) <= f.half && fabs(x - f.qx) <= f.half));
+}
+
 // ---------------------------------------------------------------- concatenated sources
 struct SrcMap {
     int nsrc;

@@ -135,11 +135,7 @@ __global__ void flap_mask_kernel(const unsigned char* __restrict__ img, unsigned
     extracted[v] = (on && inside) ? 1 : 0;                              // transforms.py:294
 }
 
-// shape_3d(shape="flap") (utilities.py:145-166): union of two cylinders along d (raster_geometry.cylinder, axis 0) and
-// a cube (raster_geometry.cube).  raster_geometry is an un-vendored, unpinned dependency of the reference and is not
-// installed here, so its published algorithm is RESTATED -- parity unpinned: relative positions become absolute grid
-// origins x0 = round((dim - 1) * rel) (round half to even), a cylinder is {(y-y0)^2 + (x-x0)^2 <= radius^2 and
-// |z-z0| <= height/2}, a cube is {|c - c0| <= side/2 on every axis}, all in float64.
+// shape_3d(shape="flap") (utilities.py:145-166): flap_hole / flap_inside (common.cuh)
 __global__ void flap_shape_mask_kernel(const unsigned char* __restrict__ img, unsigned char* __restrict__ masked,
                                        unsigned char* __restrict__ extracted, int d, int h, int w,
                                        const int* __restrict__ center, double size, double c_diam, long long nvox) {
@@ -148,19 +144,8 @@ __global__ void flap_shape_mask_kernel(const unsigned char* __restrict__ img, un
     const int x = (int)(v % w);
     const int y = (int)((v / w) % h);
     const int z = (int)(v / ((long long)w * h));
-    const double c0 = (double)center[0], c1 = (double)center[1], c2 = (double)center[2];
-    // center_relative, z_edge_1, z_edge_2 (utilities.py:148-158) -> absolute origins
-    const double z0 = rint((d - 1) * (c0 / d));
-    const double ey = rint((h - 1) * ((c1 - size / 2) / h));
-    const double ex1 = rint((w - 1) * ((c2 - size / 2) / w)), ex2 = rint((w - 1) * ((c2 + size / 2) / w));
-    const double qy = rint((h - 1) * (c1 / h)), qx = rint((w - 1) * (c2 / w));
-    const double dz = z - z0;
-    const bool in_height = fabs(dz) <= size / 2;
-    const double r2 = c_diam * c_diam, dy = y - ey;
-    const bool cyl1 = in_height && (dy * dy + (x - ex1) * (x - ex1) <= r2);
-    const bool cyl2 = in_height && (dy * dy + (x - ex2) * (x - ex2) <= r2);
-    const bool cub = in_height && fabs(y - qy) <= size / 2 && fabs(x - qx) <= size / 2;
-    const bool inside = cyl1 || cyl2 || cub;                            // mask; shape_np = 1 - mask (utilities.py:165-166)
+    const FlapHole f = flap_hole(d, h, w, (double)center[0], (double)center[1], (double)center[2], size, c_diam);
+    const bool inside = flap_inside(f, z, y, x);                        // mask; shape_np = 1 - mask (utilities.py:165-166)
     const bool on = img[v] != 0;
     masked[v] = (on && !inside) ? 1 : 0;
     extracted[v] = (on && inside) ? 1 : 0;
@@ -294,8 +279,7 @@ __global__ void hu_threshold_vec_kernel(const short* __restrict__ hu, unsigned c
     reinterpret_cast<uint4*>(out)[i] = make_uint4(o[0], o[1], o[2], o[3]);
 }
 
-// sphere / box with an INTEGER radius (np.random.randint, transforms.py:268): squared distances of integer offsets are
-// exact in int64 and sqrt is monotone, so  norm <= size  <=>  d2 <= size^2  bit for bit; 16 voxels of one row per thread
+// sphere / box with an INTEGER radius (ball_inside, common.cuh); 16 voxels of one row per thread
 template <typename I>   // I = int when every squared distance fits 31 bits (volumes up to 16384 voxels a side), else long long
 __global__ void flap_mask_vec_kernel(const unsigned char* __restrict__ img, unsigned char* __restrict__ masked,
                                      unsigned char* __restrict__ extracted, int d, int h, int w, const int* __restrict__ center,
@@ -308,15 +292,12 @@ __global__ void flap_mask_vec_kernel(const unsigned char* __restrict__ img, unsi
     const int z = (int)(i / ((long long)wg * h));
     const I size = (I)size_ll;
     const I dz = z - center[0], dy = y - center[1], cx = center[2];
-    const I base2 = dz * dz + dy * dy, size2 = size * size;
-    const bool row_in_box = (dz < 0 ? -dz : dz) <= size && (dy < 0 ? -dy : dy) <= size;
     const uint4 u = reinterpret_cast<const uint4*>(img)[i];
     const uint32_t wv[4] = {u.x, u.y, u.z, u.w};
     uint32_t m[4] = {0, 0, 0, 0}, e[4] = {0, 0, 0, 0};
 #pragma unroll
     for (int j = 0; j < 16; ++j) {
-        const I dx = x0 + j - cx;
-        const bool inside = shape == 0 ? (base2 + dx * dx <= size2) : (row_in_box && (dx < 0 ? -dx : dx) <= size);
+        const bool inside = ball_inside<I>(shape, dz, dy, x0 + j - cx, size);
         const bool on = ((wv[j >> 2] >> (8 * (j & 3))) & 0xffu) != 0;
         if (on && !inside) m[j >> 2] |= 1u << (8 * (j & 3));
         if (on && inside) e[j >> 2] |= 1u << (8 * (j & 3));
@@ -325,7 +306,7 @@ __global__ void flap_mask_vec_kernel(const unsigned char* __restrict__ img, unsi
     reinterpret_cast<uint4*>(extracted)[i] = make_uint4(e[0], e[1], e[2], e[3]);
 }
 
-// the flap shape, 16 voxels of one row per thread (same float64 arithmetic as flap_shape_mask_kernel, row terms hoisted)
+// the flap shape, 16 voxels of one row per thread (flap_hole / flap_inside, common.cuh)
 __global__ void flap_shape_mask_vec_kernel(const unsigned char* __restrict__ img, unsigned char* __restrict__ masked,
                                            unsigned char* __restrict__ extracted, int d, int h, int w,
                                            const int* __restrict__ center, double size, double c_diam, long long ngroups) {
@@ -335,22 +316,13 @@ __global__ void flap_shape_mask_vec_kernel(const unsigned char* __restrict__ img
     const int x0 = (int)(i % wg) << 4;
     const int y = (int)((i / wg) % h);
     const int z = (int)(i / ((long long)wg * h));
-    const double c0 = (double)center[0], c1 = (double)center[1], c2 = (double)center[2];
-    const double z0 = rint((d - 1) * (c0 / d));
-    const double ey = rint((h - 1) * ((c1 - size / 2) / h));
-    const double ex1 = rint((w - 1) * ((c2 - size / 2) / w)), ex2 = rint((w - 1) * ((c2 + size / 2) / w));
-    const double qy = rint((h - 1) * (c1 / h)), qx = rint((w - 1) * (c2 / w));
-    const bool in_height = fabs(z - z0) <= size / 2;
-    const double r2 = c_diam * c_diam, dy = y - ey, dy2 = dy * dy;
-    const bool cube_row = in_height && fabs(y - qy) <= size / 2;
+    const FlapHole f = flap_hole(d, h, w, (double)center[0], (double)center[1], (double)center[2], size, c_diam);
     const uint4 u = reinterpret_cast<const uint4*>(img)[i];
     const uint32_t wv[4] = {u.x, u.y, u.z, u.w};
     uint32_t m[4] = {0, 0, 0, 0}, e[4] = {0, 0, 0, 0};
 #pragma unroll
     for (int j = 0; j < 16; ++j) {
-        const double x = x0 + j;
-        const bool inside = in_height && ((dy2 + (x - ex1) * (x - ex1) <= r2) || (dy2 + (x - ex2) * (x - ex2) <= r2)) ||
-                            (cube_row && fabs(x - qx) <= size / 2);
+        const bool inside = flap_inside(f, z, y, x0 + j);
         const bool on = ((wv[j >> 2] >> (8 * (j & 3))) & 0xffu) != 0;
         if (on && !inside) m[j >> 2] |= 1u << (8 * (j & 3));
         if (on && inside) e[j >> 2] |= 1u << (8 * (j & 3));

@@ -117,18 +117,28 @@ class TrainStep:
     ``augment=utilities.RandomAffine(...)``: ``step_from_masks`` / ``step_from_bits`` draw one random affine transform per
     sample and encode the transformed masks straight into the step's inputs (``ctu_affine_encode_flaprec``; the atlas
     channel stays as it is), outside the captured graph like the plain encoders; ``last_affine()`` returns what the latest
-    step drew.  Such a step takes masks only: ``__call__`` with a ready image raises ``ValueError``."""
+    step drew.  Such a step takes masks only: ``__call__`` with a ready image raises ``ValueError``.
+
+    ``craniectomy=utilities.RandomCraniectomy(...)``: the step takes the FULL skulls only (``step_from_skulls`` /
+    ``step_from_skull_bits``) and cuts one random hole per sample on the device, fused into the same encoder launch (and
+    with ``augment`` into the same gather: the hole is cut in skull space, then transformed); ``last_craniectomy()``
+    returns the drawn holes.  ``__call__``, ``step_from_masks`` and ``step_from_bits`` take masks that are already cut and
+    raise ``ValueError`` on such a step."""
 
     def __init__(self, model, handler: str = "double", dice_lambda: float = 1.0, ce_lambda: float = 1.0,
                  lr: float = 1e-4, weight_decay: float = 0.0, optimizer: str = "adam", momentum: float = 0.99,
                  scheduler=False, grad_sync: Optional[GradSync] = None, input_requires_grad: bool = True,
-                 graph: bool = False, split_graph: Optional[bool] = None, augment=None):
-        from .utilities import RandomAffine
+                 graph: bool = False, split_graph: Optional[bool] = None, augment=None, craniectomy=None):
+        from .utilities import RandomAffine, RandomCraniectomy
         if augment is not None and not isinstance(augment, RandomAffine):
             raise TypeError("augment: a utilities.RandomAffine or None")
+        if craniectomy is not None and not isinstance(craniectomy, RandomCraniectomy):
+            raise TypeError("craniectomy: a utilities.RandomCraniectomy or None")
         self.model = model
         self.augment = augment
+        self.craniectomy = craniectomy
         self._last_affine = None                              # (params, matrices) of the latest augmenting step
+        self._last_craniectomy = None                         # params [B, 7] of the latest craniectomy step
         self.spec = _LossSpec(handler, dice_lambda, ce_lambda)
         self.handler, self.keys = handler, self.spec.keys
         self.input_requires_grad = input_requires_grad       # Model.py:351-352
@@ -200,7 +210,13 @@ class TrainStep:
         self._update(comps)
         return comps
 
+    def _no_craniectomy(self, what):
+        if self.craniectomy is not None:
+            raise ValueError("%s takes masks that are already cut: a TrainStep with craniectomy takes the full skulls "
+                             "through step_from_skulls / step_from_skull_bits" % what)
+
     def __call__(self, image: torch.Tensor, target):
+        self._no_craniectomy("__call__")
         if self.augment is not None:
             raise ValueError("an augmenting TrainStep transforms masks: feed it through step_from_masks / step_from_bits")
         return self._step(image, target)
@@ -272,6 +288,7 @@ class TrainStep:
         targets (16 bytes per voxel, read twice per step) never exist.  Without the fused head + loss, or when the step was
         captured with float targets, the one-hot targets are encoded as well."""
         from .utilities import encode_flaprec_batch
+        self._no_craniectomy("step_from_masks")
         if self.handler != "double":
             raise ValueError("step_from_masks feeds the double-output handler (full skull + flap targets)")
         masks = FUSED_HEAD_LOSS and (self._graph is None or self._static[1].dtype == torch.uint8)
@@ -301,6 +318,7 @@ class TrainStep:
         3 bits per voxel over PCIe.  ``ctu_encode_flaprec_bits`` expands them straight into the captured step's static
         inputs -- the float image (+ atlas) and the two uint8 label masks the fused head + loss kernels read."""
         from .utilities import encode_flaprec_bits
+        self._no_craniectomy("step_from_bits")
         if self.handler != "double" or not FUSED_HEAD_LOSS:
             raise ValueError("step_from_bits feeds the double-output handler through the fused head + loss kernels")
         if self.augment is not None:
@@ -314,16 +332,40 @@ class TrainStep:
         image, masks = encode_flaprec_bits(broken_bits, full_bits, flap_bits, vol_shape, atlas)
         return self._step(image, masks)
 
+    def step_from_skulls(self, full: torch.Tensor, atlas=None):
+        """One iteration from the FULL skulls of a batch (uint8 / bool [B, D, H, W] on the device, non-zero is bone):
+        ``craniectomy`` draws one hole per sample and the fused encoder writes the broken skull (+ atlas) image and the
+        full / flap label masks straight into the step's inputs -- no host synchronisation, one mask per sample."""
+        if self.craniectomy is None:
+            raise ValueError("step_from_skulls needs TrainStep(craniectomy=RandomCraniectomy(...))")
+        if self.handler != "double" or not FUSED_HEAD_LOSS:
+            raise ValueError("step_from_skulls feeds the double-output handler through the fused head + loss kernels")
+        if not isinstance(full, torch.Tensor):
+            raise TypeError("full: a uint8 [B, D, H, W] tensor")
+        return self._augmented(0, (full,), tuple(full.shape[1:]), atlas)
+
+    def step_from_skull_bits(self, full_bits: torch.Tensor, vol_shape, atlas=None):
+        """``step_from_skulls`` for BIT-PACKED full skulls ([B, D*H*W/8] uint8 on the device, ``utilities.pack_mask_bits``):
+        1 bit per voxel over PCIe."""
+        if self.craniectomy is None:
+            raise ValueError("step_from_skull_bits needs TrainStep(craniectomy=RandomCraniectomy(...))")
+        if self.handler != "double" or not FUSED_HEAD_LOSS:
+            raise ValueError("step_from_skull_bits feeds the double-output handler through the fused head + loss kernels")
+        return self._augmented(1, (full_bits,), tuple(vol_shape), atlas)
+
     def _augmented(self, bits: int, srcs, vol, atlas):
-        """Draw the batch's transforms and encode the transformed masks into the step's inputs (the captured graph's static
-        inputs once it exists): float image (+ the atlas, untransformed) and the two uint8 label masks."""
+        """Draw the batch's transforms and / or holes and encode the resulting masks into the step's inputs (the captured
+        graph's static inputs once it exists): float image (+ the atlas, untransformed) and the two uint8 label masks.
+        ``srcs``: the (broken, full, flap) masks, or with ``craniectomy`` the full skulls alone."""
         broken = srcs[0]
+        what = ("one uint8 bit-packed [B, D*H*W/8] skull batch" if len(srcs) == 1 else
+                "three uint8 bit-packed [B, D*H*W/8] masks of one shape") if bits else \
+            ("one uint8 / bool [B, D, H, W] skull batch" if len(srcs) == 1 else "three uint8 [B, D, H, W] masks of one shape")
         for t in srcs:
             if not isinstance(t, torch.Tensor) or not t.is_cuda:
                 raise RuntimeError("the masks must be CUDA tensors (no CPU fallback)")
             if t.dtype not in ((torch.uint8,) if bits else (torch.uint8, torch.bool)) or t.shape != broken.shape:
-                raise TypeError("three %s masks of one shape expected" % ("uint8 bit-packed [B, D*H*W/8]" if bits else
-                                                                         "uint8 [B, D, H, W]"))
+                raise TypeError("%s expected" % what)
         if len(vol) != 3:
             raise ValueError("vol_shape: (D, H, W)")
         b = broken.shape[0]
@@ -343,12 +385,23 @@ class TrainStep:
             image = torch.empty((b, cin, d, h, w), dtype=torch.float32, device=broken.device)
             fm = torch.empty((b, d, h, w), dtype=torch.uint8, device=broken.device)
             lm = torch.empty_like(fm)
-        params, mats = self.augment.draw(b, (d, h, w), broken.device)
         src = [t.contiguous() for t in srcs]
-        call("ctu_affine_encode_flaprec", bits, *[t.data_ptr() for t in src],
-             atlas.contiguous().data_ptr() if atlas is not None else None, mats.data_ptr(), image.data_ptr(), fm.data_ptr(),
-             lm.data_ptr(), b, cin, d, h, w, stream_ptr())
-        self._last_affine = (params, mats)
+        hole = None
+        if self.craniectomy is not None:
+            hole = self.craniectomy.draw(src[0], (d, h, w) if bits else None)
+        mats = None
+        if self.augment is not None:
+            params, mats = self.augment.draw(b, (d, h, w), broken.device)
+            self._last_affine = (params, mats)
+        atlas_ptr = atlas.contiguous().data_ptr() if atlas is not None else None
+        if hole is not None:
+            call("ctu_craniectomy_encode_flaprec", bits, src[0].data_ptr(), hole.data_ptr(), atlas_ptr,
+                 mats.data_ptr() if mats is not None else None, image.data_ptr(), fm.data_ptr(), lm.data_ptr(), b, cin, d, h,
+                 w, stream_ptr())
+            self._last_craniectomy = hole
+        else:
+            call("ctu_affine_encode_flaprec", bits, *[t.data_ptr() for t in src], atlas_ptr, mats.data_ptr(), image.data_ptr(),
+                 fm.data_ptr(), lm.data_ptr(), b, cin, d, h, w, stream_ptr())
         if self._graph is not None:
             return self._replay()
         return self._step(image, (fm, lm))
@@ -357,6 +410,10 @@ class TrainStep:
         """``(params [B, 10], matrices [B, 3, 4])`` the latest augmenting step drew (``RandomAffine.draw``), or None; valid
         until the next step."""
         return self._last_affine
+
+    def last_craniectomy(self):
+        """params [B, 7] of the holes the latest craniectomy step drew (``RandomCraniectomy.draw``), or None."""
+        return self._last_craniectomy
 
     @property
     def lr(self) -> float:

@@ -11,6 +11,8 @@
   SaltAndPepper           ctunet/pytorch/transforms.py:13-49
   RandomAffine,           no reference counterpart: seeded rotation, scaling, translation and flips of mask batches
   affine_masks            (DESIGN.md section 7e; oracle tests/affine_oracle.py)
+  RandomCraniectomy       SkullRandomHole / random_blank_patch drawn on the device from a Philox stream, without host
+                          synchronisation (DESIGN.md section 7f; oracle tests/craniectomy_oracle.py)
 
 The 'flap' shape of shape_3d calls the un-vendored, unpinned ``raster_geometry`` package in the reference
 (utilities.py:145-166); it is not installed here, so ``cylinder`` / ``cube`` are RESTATED from the package's published
@@ -526,4 +528,99 @@ class RandomAffine(object):
             res["target"] = type(tgt)(out[1:])
         elif tgt is not None:
             res["target"] = out[1]
+        return res
+
+
+# ---------------------------------------------------------------------------------------------- RandomCraniectomy
+CRANIECTOMY_DOMAIN = 0xC4A1       # engine.philox_key domain of the craniectomy draws
+CRANIECTOMY_PARAM_KEYS = ("applied", "shape", "radius", "c_diam", "z", "y", "x")
+
+
+class RandomCraniectomy(object):
+    """The virtual craniectomy drawn and cut on the device (DESIGN.md section 7f): per sample the distribution of
+    ``random_blank_patch(full, p, True, p_type="random", valid_shapes=shapes)`` (transforms.py:241-300) -- a gate
+    ``u <= p``, a centre uniform over the skull's bone voxels, an integer radius uniform in ``radius_bounds``, a shape
+    uniform over ``shapes`` (sphere, box, flap) and the flap's cylinder radius -- drawn from a Philox stream on the device
+    instead of the host RNGs, so nothing synchronises with the host.  ``random_blank_patch`` / ``SkullRandomHole`` replay
+    the reference's host draws; this transform has the same distribution, not the same stream.
+
+    The key is ``engine.philox_key(device, CRANIECTOMY_DOMAIN)`` when the transform first draws on a device and the pass
+    counter lives in device memory (as ``RandomAffine``): ``torch.manual_seed(s)`` before the first draw reproduces a run.
+
+    ``__call__(sample)`` is the sync-free twin of ``SkullRandomHole(p, double_output=True)``: a uint8 / bool CUDA
+    ``image`` [B, D, H, W] or [D, H, W] (the full skull, non-zero is bone) gives ``{"image": broken, "target": (full,
+    flap)}`` as uint8, with ``broken & flap == 0`` and ``broken | flap == full``; ``RandomAffine()(RandomCraniectomy()(s))``
+    composes.  ``TrainStep(craniectomy=...)`` fuses the cut into the batch encoding of the training step."""
+
+    def __init__(self, p=1.0, shapes=("sphere", "box", "flap")):
+        if not _number(p) or not 0 <= p <= 1:
+            raise ValueError("p must be in [0, 1], got %r" % (p,))
+        if isinstance(shapes, str) or not isinstance(shapes, (tuple, list)) or not shapes or \
+                not all(isinstance(s, str) and s in _SHAPES for s in shapes):
+            raise ValueError("shapes: a non-empty list of 'sphere', 'box', 'flap', got %r" % (shapes,))
+        self.p = float(p)
+        self.shapes = tuple(shapes)
+        self._shape_bits = sum({1 << _SHAPES[s] for s in shapes})
+        self._state = {}                   # device -> (key, int64 pass counter on the device)
+        self.last = None                   # params [B, 7] of the latest draw
+
+    def _full(self, full, vol_shape):
+        """Validate the full skulls (errors before any launch) -> (bits, contiguous tensor, batch, (d, h, w), radius range)."""
+        if not isinstance(full, torch.Tensor):
+            raise TypeError("RandomCraniectomy expects a tensor, got %s" % type(full).__name__)
+        if vol_shape is None:
+            if full.dtype not in (torch.uint8, torch.bool):
+                raise TypeError("RandomCraniectomy expects uint8 or bool skull masks, got %s" % full.dtype)
+            if full.dim() not in (3, 4):
+                raise ValueError("RandomCraniectomy expects [B, D, H, W] or [D, H, W] masks, got %s" % (tuple(full.shape),))
+            bits, vol = 0, tuple(int(v) for v in full.shape[-3:])
+            batch = full.shape[0] if full.dim() == 4 else 1
+        else:
+            vol = tuple(int(v) for v in vol_shape)
+            if len(vol) != 3:
+                raise ValueError("vol_shape: (D, H, W)")
+            if full.dtype != torch.uint8 or full.dim() != 2 or full.shape[1] * 8 != vol[0] * vol[1] * vol[2]:
+                raise ValueError("bit-packed skulls: uint8 [B, D*H*W/8] of the volume shape %s, got %s %s"
+                                 % (vol, full.dtype, tuple(full.shape)))
+            bits, batch = 1, full.shape[0]
+        if not 1 <= batch <= 65535 or not all(1 <= v <= 16384 for v in vol):
+            raise ValueError("RandomCraniectomy: batch 1..65535 and axes 1..16384, got %d x %s" % (batch, vol))
+        min_r, max_r = (int(r) for r in radius_bounds(vol))
+        if min_r >= max_r:                 # np.random.randint(min_r, max_r) raises in the reference
+            raise ValueError("the radius range [%d, %d) of a %s volume is empty" % (min_r, max_r, vol))
+        if not full.is_cuda:
+            raise RuntimeError("RandomCraniectomy runs on CUDA tensors only (no CPU fallback)")
+        return bits, full.contiguous(), batch, vol, (min_r, max_r)
+
+    def draw(self, full: torch.Tensor, vol_shape=None) -> torch.Tensor:
+        """Draw one hole per sample of ``full`` (uint8 / bool [B, D, H, W] or [D, H, W]; with ``vol_shape`` bit-packed
+        [B, D*H*W/8], ``pack_mask_bits``): float64 CUDA params [B, 7] = ``CRANIECTOMY_PARAM_KEYS`` (applied 0 / 1, shape
+        0 sphere / 1 box / 2 flap, radius, c_diam (flap; 0 otherwise), the centre voxel z, y, x (-1 when not applied)).
+        No host synchronisation."""
+        bits, src, batch, vol, (min_r, max_r) = self._full(full, vol_shape)
+        device = src.device
+        st = self._state.get(device)
+        if st is None:
+            from .engine import philox_key
+            st = self._state[device] = (philox_key(device, CRANIECTOMY_DOMAIN), torch.zeros(1, dtype=torch.int64, device=device))
+        with torch.cuda.device(device):
+            nbytes = _load().ctu_craniectomy_workspace_bytes(batch, *vol)
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
+            params = torch.empty((batch, 7), dtype=torch.float64, device=device)
+            call("ctu_craniectomy_draw", bits, src.data_ptr(), batch, *vol, self.p, self._shape_bits, min_r, max_r, st[0],
+                 st[1].data_ptr(), params.data_ptr(), ws.data_ptr(), nbytes, stream_ptr())
+        self.last = params
+        return params
+
+    def __call__(self, sample):
+        img = sample["image"]
+        _, full, batch, vol, _ = self._full(img, None)
+        params = self.draw(full)
+        u8 = full.view(torch.uint8) if full.dtype == torch.bool else full      # bool is one byte of 0 / 1
+        out = [torch.empty(u8.shape, dtype=torch.uint8, device=u8.device) for _ in range(3)]
+        with torch.cuda.device(u8.device):
+            call("ctu_craniectomy_masks_u8", u8.data_ptr(), params.data_ptr(), *[t.data_ptr() for t in out], batch, *vol,
+                 stream_ptr())
+        res = dict(sample)
+        res["image"], res["target"] = out[0], (out[1], out[2])
         return res

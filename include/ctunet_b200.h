@@ -451,6 +451,37 @@ int ctu_affine_encode_flaprec(int bits, const unsigned char* broken, const unsig
 int ctu_affine_masks_u8(int n, const unsigned char* const* h_src, unsigned char* const* h_dst, const float* matrices,
                         int batch, int d, int h, int w, ctu_stream stream);
 
+/* ---- virtual craniectomy drawn on the device (DESIGN.md section 7f): per sample the distribution of
+ *      random_blank_patch(full, p, True, p_type="random", valid_shapes) (transforms.py:241-300) from a Philox stream
+ *      instead of the host RNGs.  full = the full-skull masks, uint8 [batch][d][h][w] (bits = 0; non-zero is bone) or
+ *      bit-packed [batch * d*h*w / 8] (bits = 1, as ctu_encode_flaprec_bits); 1 <= batch <= 65535, every axis 1..16384.
+ *      params = DEVICE double[batch][7] (applied, shape, radius, c_diam, z, y, x): shape 0 sphere / 1 box / 2 flap as
+ *      ctu_flap_mask_u8, the integer radius, c_diam for the flap (0 otherwise), the centre voxel (-1s when not applied).
+ *      params is 8-byte aligned; `full` has no alignment requirement (a bit-packed view may start at any byte).
+ *      Philox4x32-10 with key = seed and counter = (pass, sample, call); the words r[call][0..3] feed:
+ *        call 0: gate u = u53(r0, r1) (applied iff u <= p and the skull has bone), k = floor((r2 | r3 << 32) * n / 2^64)
+ *                -> centre = np.argwhere(full > 0)[k] (n bone voxels, C order)
+ *        call 1: radius = min_radius + floor((r0 | r1 << 32) * (max_radius - min_radius) / 2^64); shape = the enabled
+ *                shape (bit 0 sphere, 1 box, 2 flap of `shapes`) of rank floor((r2 | r3 << 32) * popcount(shapes) / 2^64)
+ *        call 2: c_diam = ((0.25 + 0.75 u53(r0, r1)) * radius) / 4 (flap only)
+ *      with u53(a, b) = ((a >> 5) 2^26 + (b >> 6)) / 2^53.  ws: DEVICE scratch of ctu_craniectomy_workspace_bytes bytes,
+ *      16-byte aligned (-1: invalid shape).  Two launches (per-chunk bone counts, then one CTA for the batch);
+ *      pass_counter: DEVICE int64 read, then advanced (NULL: pass 0).  min_radius < max_radius, 0 <= p <= 1. */
+long long ctu_craniectomy_workspace_bytes(int batch, int d, int h, int w);
+int ctu_craniectomy_draw(int bits, const unsigned char* full, int batch, int d, int h, int w, double p, int shapes,
+                         int min_radius, int max_radius, unsigned long long seed, unsigned long long* pass_counter,
+                         double* params, void* ws, long long ws_bytes, ctu_stream stream);
+/* ctu_affine_encode_flaprec from the full skull alone, the hole cut in source space: for output voxel p with source voxel s
+ * (matrices as ctu_affine_encode_flaprec, or NULL: s = p), full = (full[s] != 0), inside = the hole of params (as
+ * ctu_craniectomy_draw writes them) at s with the arithmetic of ctu_flap_mask_u8; image channel 0 = full AND NOT inside as
+ * float, channel 1 = the atlas unchanged, full_mask = full, flap_mask = full AND inside (uint8). */
+int ctu_craniectomy_encode_flaprec(int bits, const unsigned char* full, const double* params, const float* atlas,
+                                   const float* matrices, float* image, unsigned char* full_mask, unsigned char* flap_mask,
+                                   int batch, int in_channels, int d, int h, int w, ctu_stream stream);
+/* the same cut as uint8 masks, no transform: broken = full AND NOT inside, full_out = full, flap = full AND inside */
+int ctu_craniectomy_masks_u8(const unsigned char* full, const double* params, unsigned char* broken, unsigned char* full_out,
+                             unsigned char* flap, int batch, int d, int h, int w, ctu_stream stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
