@@ -833,6 +833,11 @@ static int head_loss_setup(HeadParams& p, int flags, int cout, const void* tgt0,
     CTU_REQUIRE(tgt0 && (pairs == 1 || tgt1) && sums, "%s: missing target / sums", what);
     CTU_REQUIRE(ce_lambda != 0.f || dice_lambda != 0.f, "%s: both loss weights are zero", what);
     CTU_REQUIRE(pairs == 2 || cout >= 2 || ce_lambda == 0.f, "%s: CrossEntropy needs at least two classes", what);
+    // head_load_targets2 reads two voxels per load (uchar2 / float2): a target view at an odd byte (uint8) or 4-mod-8 byte
+    // (float) offset would fault inside the kernel
+    const uintptr_t talign = target_u8 ? 2 : 8;
+    CTU_REQUIRE(reinterpret_cast<uintptr_t>(tgt0) % talign == 0 && reinterpret_cast<uintptr_t>(tgt1) % talign == 0,
+                "%s: %s targets must be %d-byte aligned", what, target_u8 ? "uint8" : "float32", (int)talign);
     p.tgt0 = reinterpret_cast<const float*>(tgt0); p.tgt1 = reinterpret_cast<const float*>(tgt1); p.lsums = sums;
     p.softmax_for_dice = softmax_for_dice; p.want_ce = ce_lambda != 0.f;
     p.g_ce = ce_lambda; p.g_dice = dice_lambda;
@@ -1149,6 +1154,7 @@ int ctu_head_loss_bwd(int dtype, const void* const* h_srcs, const int* h_src_cha
                          dice_lambda, pairs, "ctu_head_loss_bwd");
     if (rc != CTU_OK) return rc;
     CTU_REQUIRE(h_dsrcs != nullptr && dlogits != nullptr, "ctu_head_loss_bwd: missing output buffers");
+    CTU_REQUIRE(reinterpret_cast<uintptr_t>(dlogits) % 8 == 0, "ctu_head_loss_bwd: dlogits must be 8-byte aligned (float2 stores)");
     for (int i = 0; i < nsrc; ++i) p.dsrc[i] = h_dsrcs[i];
     p.out0 = dlogits;
     cudaStream_t st = (cudaStream_t)stream;

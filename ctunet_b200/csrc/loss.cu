@@ -192,6 +192,12 @@ __global__ void argmax_kernel(const float* __restrict__ x, float* __restrict__ o
     out[i] = (float)bi;
 }
 
+// spatial % 4 == 0 selects the float4 path of the kernels above: every plane then starts 16-byte aligned iff the base does
+static bool vec4_aligned(long long spatial, const void* a, const void* b, const void* c = nullptr) {
+    const auto mis = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) != 0; };
+    return spatial % 4 != 0 || !(mis(a) || mis(b) || mis(c));
+}
+
 static int loss_grid(long long spatial) {
     long long g = (spatial + kLossThreads - 1) / kLossThreads;
     const long long cap = 148 * 4;
@@ -208,6 +214,7 @@ int ctu_dice_ce_fwd(const float* pred, const float* target, int b, int c, long l
                     int want_ce, double* sums, float* out, ctu_stream stream) {
     CTU_REQUIRE(pred && target && sums && out && b > 0 && c >= 1 && c <= 4 && spatial > 0,
                 "ctu_dice_ce_fwd: bad arguments (1 <= c <= 4)");
+    CTU_REQUIRE(vec4_aligned(spatial, pred, target), "ctu_dice_ce_fwd: pred and target must be 16-byte aligned (float4 loads)");
     cudaStream_t st = (cudaStream_t)stream;
     cudaError_t e = cudaMemsetAsync(sums, 0, sizeof(double) * 4 * b, st);
     if (e != cudaSuccess) {
@@ -229,6 +236,8 @@ int ctu_dice_ce_bwd(const float* pred, const float* target, int b, int c, long l
                     int want_ce, const double* sums, const float* g, float* dpred, ctu_stream stream) {
     CTU_REQUIRE(pred && target && sums && g && dpred && b > 0 && c >= 1 && c <= 4 && spatial > 0,
                 "ctu_dice_ce_bwd: bad arguments (1 <= c <= 4)");
+    CTU_REQUIRE(vec4_aligned(spatial, pred, target, dpred),
+                "ctu_dice_ce_bwd: pred, target and dpred must be 16-byte aligned (float4 loads / stores)");
     cudaStream_t st = (cudaStream_t)stream;
     dim3 grid(loss_grid(spatial) * 4, b);
     switch (c) {

@@ -1085,6 +1085,10 @@ class Engine:
                     or t.device != s0.buf.device):
                 raise TypeError("targets: contiguous float32 one-hot tensors [B, C, D, H, W] or uint8 label masks [B, D, H, W] "
                                 "on %s (expected shape %s)" % (s0.buf.device, want))
+            if t.data_ptr() % (2 if u8 else 8):
+                # the kernels read two voxels per load (csrc/head.cu, head_load_targets2)
+                raise TypeError("targets: a %s target must start %d-byte aligned (a contiguous view at offset %d elements "
+                                "is not)" % (t.dtype, 2 if u8 else 8, t.storage_offset()))
         pa, ca, ns = self._src_args(srcs)
         t0, t1 = targets[0].data_ptr(), (targets[1].data_ptr() if sp else None)
         sums = self.f64(4 * len(targets) * s0.n)

@@ -121,6 +121,7 @@ def test_bn_relu_drop_fwd_bwd(mode, fold, pool, shape, monkeypatch):
     y = eng.pack(x.to(DEV))
     res = eng.bn_relu(y, bn_gpu, True, extra_updates=0, pool=pool, keep=keep.to(DEV))
     res = res if pool else (res,)
+    ss = res[0].bn["ss"].clone()            # the fp32 scale / shift / mean / invstd the kernels use
     for o, r, nm in zip(res, outs_r, ["a", "pooled"]):
         _close(eng.unpack(o), r, mode, what=nm)
     # batch statistics are those of y (BatchNorm precedes the dropout)
@@ -132,9 +133,13 @@ def test_bn_relu_drop_fwd_bwd(mode, fold, pool, shape, monkeypatch):
     dyo = eng.unpack(eng.agrads[id(y)]).cpu()
     assert float(dyo[:, 0].abs().max()) == 0.0                         # the dropped channel passes no gradient
     if mode == "bf16" and pool:
-        # (ties of bf16-rounded values may elect a neighbouring arg-max: see tests/test_gpu_ops.py)
-        bad = ((dyo - xr.grad).abs() > 1.2e-2 * xr.grad.abs().max()).float().mean().item()
-        assert bad < 0.03, "fraction of mismatching dy elements %.4f" % bad
+        # routing exact except at windows within fp32 rounding of a flip (see tests/test_gpu_ops.py)
+        import norm_head_oracle as NO
+        cpad = (c + 7) // 8 * 8
+        ss4 = tuple(ss.double().view(4, cpad)[:, :c].cpu())
+        ref, err, gate, tie = NO.dy_error_with_ties(x, ss4, gr[0], gr[1], keep[:, :c], dyo)
+        print("tie-marked: %d gates, %d windows" % (int(gate.sum()), int(tie.sum())))
+        assert float(err.max()) <= 1.2e-2 * float(ref["dy"].abs().max()), "dy: max abs err %.3e" % float(err.max())
     else:
         _close(dyo, xr.grad, mode, what="dy")
     _close(eng.pgrads[id(bn_gpu.weight)], bn_ref.weight.grad, mode, what="dgamma")

@@ -149,6 +149,7 @@ def test_bn_relu_pool_fwd_bwd(mode, pool, shape):
     y = eng.pack(x.to(DEV))
     res = eng.bn_relu(y, bn_gpu, True, extra_updates=1, pool=pool)
     res = res if pool else (res,)
+    ss = res[0].bn["ss"].clone()            # the fp32 scale / shift / mean / invstd the kernels use
     for o, r, nm in zip(res, outs_r, ["a", "pooled"]):
         _close(eng.unpack(o), r, mode, what=nm)
     # running stats after the forward update
@@ -159,11 +160,15 @@ def test_bn_relu_pool_fwd_bwd(mode, pool, shape):
         eng.agrads[id(o)] = eng.pack(gg.to(DEV))
     eng.run_tape()
     if mode == "bf16" and pool:
-        # two window entries that round to the same bf16 value may elect a different arg-max than fp32:
-        # the routed gradient then lands on the neighbouring voxel (isolated elements, sums unaffected)
-        dyo, dyr = eng.unpack(eng.agrads[id(y)]).cpu(), xr.grad
-        bad = ((dyo - dyr).abs() > 1.2e-2 * dyr.abs().max()).float().mean().item()
-        assert bad < 0.03, "fraction of mismatching dy elements %.4f" % bad
+        # the routing of every window against float64 with the kernel's fp32 scale / shift: exact, except at windows
+        # whose arg-max lies within fp32 rounding of flipping (either child is accepted there; counted)
+        import norm_head_oracle as NO
+        cpad = (c + 7) // 8 * 8
+        ss4 = tuple(ss.double().view(4, cpad)[:, :c].cpu())
+        dyo = eng.unpack(eng.agrads[id(y)]).cpu()
+        ref, err, gate, tie = NO.dy_error_with_ties(x, ss4, gr[0], gr[1], None, dyo)
+        print("tie-marked: %d gates, %d windows" % (int(gate.sum()), int(tie.sum())))
+        assert float(err.max()) <= 1.2e-2 * float(ref["dy"].abs().max()), "dy: max abs err %.3e" % float(err.max())
     else:
         _close(eng.unpack(eng.agrads[id(y)]), xr.grad, mode, what="dy")
     _close(eng.pgrads[id(bn_gpu.weight)], bn_ref.weight.grad, mode, what="dgamma")
